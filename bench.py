@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the point-set-distance hot path (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -11,13 +11,21 @@ Workload (BASELINE.json configs[1], the configuration the metric is quoted on):
     (grad_xyz1, grad_xyz2) over one batch: two kernel launches, no memset.  metric = directed point pairs per second = 2*B*N*M / t(step), whole
     job (all ranks).  Weak scaling: every rank owns its own batch of B clouds, no data-path collective.
 
-`value`       : the shape of a training loop -- ONE step at a time, every launch on all SMs.  K steps captured in one CUDA
-                graph, replayed REPLAYS times; every replay is timed on its own with CUDA events on the launch stream (a
-                barrier + synchronise before and after, L2 flushed in between); value = K steps / MEDIAN replay time (max over
-                ranks per replay).  Batches rotate through a pool larger than L2.
-`value_pipelined`: the same steps with 8 independent batches in flight (step s on chain s % 8, every tensor-core NN launch
-                limited to a quarter of the SMs): throughput of a caller that can supply that concurrency (evaluation over many
-                batches, a pipelined host loop) -- reported next to `value`, never instead of it.
+`value`       : the shape of a training loop -- ONE step at a time, every launch on all SMs.  Exactly K = --steps timed steps,
+                captured in consecutive CUDA graphs (up to REPLAYS of them, at least MIN_REPLAY_STEPS steps each when K
+                allows), each replayed once untimed and then once timed with CUDA events on the launch stream (a barrier +
+                synchronise before and after, L2 flushed in between; WARM_REPLAYS warm-up replays of the first graph
+                right before, outside the result); value = 1 step / MEDIAN per-step time of the timed replays (max over
+                ranks per replay) -- at the default --steps 400, 4 timed replays of 100 steps.
+                Batches rotate through a pool larger than L2.
+--dump-outputs DIR: after the timed steps of `value`, rank 0 writes what its last step returned to a caller of
+                chamfer_3DDist forward + backward -- dist1, dist2, idx1, idx2 [B, N|M] and grad_xyz1, grad_xyz2 [B, N|M, 3] --
+                as DIR/<name>.npy in float32 (2.6 MB).  The inputs are seeded, so two builds run with the same arguments can
+                be compared output for output (gradients accumulate with float atomics: compare them with a tolerance).
+`value_pipelined`: the same steps, K rounded up to a multiple of 8 and timed the same way, with 8 independent batches in
+                flight (step s on chain s % 8, every tensor-core NN launch limited to a quarter of the SMs): throughput of a
+                caller that can supply that concurrency (evaluation over many batches, a pipelined host loop) -- reported
+                next to `value`, never instead of it.
 `e2e`         : the same metric through the C ABI's host-buffer step (pinned host clouds -> H2D -> forward -> fused mean
                 loss -> backward -> loss read on the host), pipelined over 8 streams, over max(K, 1000) steps (median of 3
                 runs); `e2e.gt_only` is the reference loop's real shape (train.py:160-163): the prediction is the
@@ -45,24 +53,42 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as the build left it (it may be read-only)
 
 B, N, M = 32, 2048, 2048
 EMD_EPS, EMD_ITERS = 0.005, 50
 C5_B, C5_N = 8, 131072
 NOMINAL_FP32_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12  # 74.45
-REPLAYS = 20
+REPLAYS = 20               # at most this many timed graph replays per leg (their median is reported) ...
+MIN_REPLAY_STEPS = 100     # ... of at least this many steps each, so that a graph's launch stays a small part of its time
+WARM_REPLAYS = 3           # warm-up replays right before the timed ones, outside the result (time_replays)
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=400)
+    ap.add_argument("--steps", type=int, default=400, help="timed steps of the headline measurement (`value`)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip emd / reference_cuda / cpu baselines / c4 / c5")
     ap.add_argument("--no-c4", action="store_true", help="skip the train-step leg (BASELINE configs[3])")
     ap.add_argument("--no-c5", action="store_true", help="skip the large-cloud leg (BASELINE configs[4])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32; GPU path only)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
+    return args
+
+
+def replay_lengths(total, grain=1):
+    """Split `total` timed steps into consecutive CUDA graphs, one timed replay each: up to REPLAYS graphs of at least
+    MIN_REPLAY_STEPS steps (one graph when total is smaller), every length a multiple of `grain` (total must be one)."""
+    r = max(1, min(REPLAYS, total // MIN_REPLAY_STEPS))
+    base = total // r // grain * grain
+    return [base] * (r - 1) + [total - base * (r - 1)]
 
 
 class ClockSampler(threading.Thread):
@@ -263,7 +289,7 @@ def main():
     pkg = psd_b200.load()
     L = pkg._lib
     lib = L.lib
-    K, W = max(1, args.steps), max(args.warmup, 3)
+    K, W = args.steps, max(args.warmup, 3)
 
     def barrier():
         if dist is not None:
@@ -344,41 +370,66 @@ def main():
                 stream.wait_stream(sd)
         return gr
 
-    def time_replays(gr, replays, sampler=None):
-        """Per-replay device times (ms): barrier + synchronise on both sides of every replay, L2 flushed in between."""
-        times = []
-        for _ in range(replays):
-            with torch.cuda.stream(stream):
-                flush_l2()
-            barrier()
-            with torch.cuda.stream(stream):
-                times.append(event_time_ms(torch, gr.replay, stream))
-            barrier()
-        return max_over_ranks(times)
+    def capture_split(capture, lengths, first):
+        """Consecutive graphs of `lengths` steps starting at step `first`: [(graph, steps)]."""
+        graphs = []
+        for n in lengths:
+            graphs.append((capture(n, step, first), n))
+            first += n
+        return graphs
+
+    def replay_ms(gr):
+        """One replay: L2 flushed, barrier + synchronise on both sides, CUDA events on the launch stream."""
+        with torch.cuda.stream(stream):
+            flush_l2()
+        barrier()
+        with torch.cuda.stream(stream):
+            t = event_time_ms(torch, gr.replay, stream)
+        barrier()
+        return t
+
+    def time_replays(graphs):
+        """Per-step device times (ms), max over ranks per replay: (warm-up, timed).  The first graph is replayed
+        WARM_REPLAYS times the same way first -- the first replays after a pause of the host loop run slower (their own
+        times are reported as config.warmup_replay_step_ms, outside the result) --, then every graph once."""
+        seq = [graphs[0]] * WARM_REPLAYS + graphs
+        per_step = [t / n for t, (_, n) in zip(max_over_ranks([replay_ms(gr) for gr, _ in seq]), seq)]
+        return per_step[:WARM_REPLAYS], per_step[WARM_REPLAYS:]
 
     with torch.cuda.stream(stream):
         for s in range(W):  # untimed warm-up (also loads the module before graph capture)
             step(s)
         stream.synchronize()
         lib.psd_chamfer_tc_ctas(0)
-        g_serial = capture_serial(K, step, W)
+        g_serial = capture_split(capture_serial, replay_lengths(K), W)
         lib.psd_chamfer_tc_ctas(TC_CTAS)
-        g_chains = capture_chains(Kp, step, W)
+        g_chains = capture_split(capture_chains, replay_lengths(Kp, CHAINS), W)
         lib.psd_chamfer_tc_ctas(0)
-        g_serial.replay(); g_chains.replay()      # one untimed replay each
+        for gr, _ in g_serial + g_chains:      # one untimed replay each
+            gr.replay()
         stream.synchronize()
 
     sampler = ClockSampler(device_index_for_nvml(local_rank))
     sampler.start()
-    t_serial = time_replays(g_serial, REPLAYS)
-    t_chains = time_replays(g_chains, REPLAYS)
+    warm_serial, t_serial = time_replays(g_serial)
+    if args.dump_outputs and rank == 0:
+        # the last timed step, W + K - 1, wrote its outputs to batch slot p; later legs reuse the slots
+        p = (W + K - 1) % pool
+        dump = {"dist1": d1[p], "dist2": d2[p], "idx1": i1[p], "idx2": i2[p],
+                "grad_xyz1": gbuf[p][: 3 * B * N].view(B, N, 3), "grad_xyz2": gbuf[p][3 * B * N:].view(B, M, 3)}
+        dump = {k: v.cpu().numpy().astype(np.float32) for k, v in dump.items()}
+    _, t_chains = time_replays(g_chains)
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, v in dump.items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
     ms_serial = statistics.median(t_serial)
     ms_chains = statistics.median(t_chains)
     pairs_step = 2.0 * B * N * M
-    value = world * pairs_step * K / (ms_serial * 1e-3)
-    value_pipelined = world * pairs_step * Kp / (ms_chains * 1e-3)
+    value = world * pairs_step / (ms_serial * 1e-3)
+    value_pipelined = world * pairs_step / (ms_chains * 1e-3)
 
     # ---- end to end through the C ABI's host-buffer entry points of the path's caller, Loss.get_chamfer_loss + backward
     # (loss/loss.py:30-37): pinned host clouds -> H2D -> forward -> fused mean loss -> backward -> loss on the host
@@ -444,16 +495,18 @@ def main():
 
     out = {
         "metric": "chamfer_fwd_bwd_point_pairs_per_s", "value": value, "unit": "pairs/s", "n_gpus": world, "steps": K,
-        "warmup": W, "ms_per_step": ms_serial / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+        "warmup": W, "ms_per_step": ms_serial, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic",
-        "value_pipelined": {"value": value_pipelined, "unit": "pairs/s", "steps": Kp, "ms_per_step": ms_chains / Kp,
+        "value_pipelined": {"value": value_pipelined, "unit": "pairs/s", "steps": Kp, "ms_per_step": ms_chains,
                             "chains": CHAINS, "tc_ctas_per_launch": TC_CTAS,
-                            "what": f"{CHAINS} independent batches in flight (step s on chain s % {CHAINS} of one graph), every tensor-core NN launch limited to {TC_CTAS} CTAs; same replay protocol as `value`"},
+                            "what": f"{CHAINS} independent batches in flight (step s on chain s % {CHAINS} of its graph), every tensor-core NN launch limited to {TC_CTAS} CTAs; same replay protocol as `value`"},
         "config": {"workload": f"chamfer3D fwd+bwd B={B} per GPU, N=M={N}, fp32, bit-exact idx (BASELINE configs[1])",
                    "cache": f"inputs larger than L2: {pool} batches x {per_batch / 1e6:.1f} MB rotate, one per step; L2 flushed (256 MB write) before every timed replay",
-                   "timing": f"`value`: one step at a time (forward launch on all SMs as a programmatic dependent of the previous backward, then the backward as a plain launch), K steps captured in one CUDA graph; {REPLAYS} replays, each bracketed by barrier + synchronise and timed with CUDA events on the launch stream; median replay (max over ranks per replay)",
-                   "replay_ms_min_median_max": [min(t_serial), ms_serial, max(t_serial)],
-                   "timed_steps_total": K * REPLAYS,
+                   "timing": f"`value`: one step at a time (forward launch on all SMs as a programmatic dependent of the previous backward, then the backward as a plain launch), the K timed steps captured in {len(g_serial)} consecutive CUDA graph(s); each replayed once untimed, then (after {WARM_REPLAYS} warm-up replays of the first graph, outside the result) once bracketed by barrier + synchronise and timed with CUDA events on the launch stream; median per-step time over the {len(g_serial)} timed replay(s) (max over ranks per replay)",
+                   "replay_steps": [n for _, n in g_serial],
+                   "step_ms_min_median_max": [min(t_serial), ms_serial, max(t_serial)],
+                   "warmup_replay_step_ms": warm_serial,
+                   "timed_steps_total": K,
                    "parallelism": f"batch-sharded x{world}, no data-path collective"},
         "e2e": {"value": e2e_value, "unit": "pairs/s", "h2d_bytes_per_step": 4 * 3 * B * (N + M), "d2h_bytes_per_step": 4,
                 "steps": Ke, "ms_per_step": t_pipe / Ke, "pipeline_depth": DEPTH, "tc_ctas_per_launch": TC_CTAS,
@@ -463,7 +516,7 @@ def main():
                             "api": "psd_chamfer_loss_step_pred_dev: the training loop's real shape (train.py:160-163) -- the prediction is the generator's [B,3,N] device tensor (read in place), only the ground truth crosses PCIe; d loss / d pred stored in the prediction's layout on the device"},
                 "synchronous": {"value": world * pairs_step * 200 / (t_sync * 1e-3), "unit": "pairs/s", "api": "psd_chamfer_loss_step_host: the same step, one blocking call per step (no overlap)"},
                 "torch_api": {"value": world * pairs_step * 100 / (t_torch * 1e-3), "unit": "pairs/s", "api": "Loss().get_chamfer_loss(pred, gt); loss.backward(); loss.item() with a pinned-host H2D copy per step"}},
-        "gpu_launches": 2 * K * REPLAYS,   # value leg: chamfer_nn_tc_kernel + chamfer_grad_kernel per step
+        "gpu_launches": 2 * K,   # value leg: chamfer_nn_tc_kernel + chamfer_grad_kernel per timed step
         "clocks": sampler.result(),
     }
 
