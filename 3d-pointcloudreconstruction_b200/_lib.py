@@ -34,6 +34,9 @@ _SIGNATURES = {
     "psd_emd_forward_cluster": [_vp, _vp, _ci, _ci, _vp, _vp, _vp, _vp, _cf, _ci, _ci, _vp],
     "psd_emd_backward": [_vp, _vp, _vp, _vp, _vp, _ci, _ci, _vp],
     "psd_emd_backward_ex": [_vp, _vp, _vp, _vp, _vp, _ci, _ci, _ci, _vp],
+    "psd_emd_dual_bound": [_vp, _vp, _ci, _ci, _vp, _vp, _vp, _vp, _vp],
+    "psd_emd_certified": [_vp, _vp, _ci, _ci, _cf, _cf, _cf, _ci, _vp, _vp, _vp, _vp, _vp, _vp],
+    "psd_emd_certified_cluster": [_vp, _vp, _ci, _ci, _cf, _cf, _cf, _ci, _vp, _vp, _vp, _vp, _vp, _ci, _vp],
     "psd_emd_mean_loss_forward": [_vp, _vp, _ci, _ci, _vp, _vp, _cf, _ci, _vp, _vp, _vp],
     "psd_emd_mean_loss_backward": [_vp, _vp, _vp, _vp, _vp, _vp, _ci, _ci, _vp],
     "psd_chamfer_forward_host": [_vp, _vp, _ci, _ci, _ci, _vp, _vp, _vp, _vp, _vp],

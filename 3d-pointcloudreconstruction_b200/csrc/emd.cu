@@ -1038,6 +1038,140 @@ __global__ void emd_mean_loss_kernel(const float *__restrict__ sums, int b, floa
     if (threadIdx.x == 0) *out = __fdiv_rn(s1, (float)b);
 }
 
+// ---- Certificate of an (assignment, prices) pair: weak-duality bounds on the Euclidean EMD (emd_certified).
+// For ANY prices p and any permutation a:  sum_j d(j, a_j)  >=  L = sum_j min_k (d_jk + p_k) - sum_k p_k,  and U = sum_j d(j, a_j)
+// is the cost of a feasible matching, so L <= optimum <= U.  Nothing about the auction is assumed.  Every quantity is
+// rounded towards its bound: d_jk + p_k downwards for L (|dx| rounded down, squares and sums of squares rounded down,
+// __dsqrt_rd), sum_k p_k upwards; d(j, a_j) upwards for U.  The sums run in a fixed order (no float atomics): the bounds are
+// reproducible bit for bit.
+constexpr int kBoundThreads = 256;
+constexpr int kBoundRowsPerLane = 8;                                   // bidders per warp; every lane carries all of them
+constexpr int kBoundRows = (kBoundThreads / 32) * kBoundRowsPerLane;   // 64 bidders per CTA
+constexpr int kBoundTile = 2048;                                       // objects staged in shared memory per pass (32 KB)
+
+// |a - b| of two floats rounded down / up in fp64 (the exact difference of two floats does not always fit a double)
+__device__ __forceinline__ double absdiff_rd(float a, float b) { return __dsub_rd((double)fmaxf(a, b), (double)fminf(a, b)); }
+__device__ __forceinline__ double absdiff_ru(float a, float b) { return __dsub_ru((double)fmaxf(a, b), (double)fminf(a, b)); }
+__device__ __forceinline__ double sqdist_rd(float ax, float ay, float az, float bx, float by, float bz) {
+    const double dx = absdiff_rd(ax, bx), dy = absdiff_rd(ay, by), dz = absdiff_rd(az, bz);
+    return __fma_rd(dz, dz, __fma_rd(dy, dy, __dmul_rd(dx, dx)));
+}
+__device__ __forceinline__ double sqdist_ru(float ax, float ay, float az, float bx, float by, float bz) {
+    const double dx = absdiff_ru(ax, bx), dy = absdiff_ru(ay, by), dz = absdiff_ru(az, bz);
+    return __fma_ru(dz, dz, __fma_ru(dy, dy, __dmul_ru(dx, dx)));
+}
+
+// CTA (blockIdx.x, cloud blockIdx.y) owns 64 bidders j: part_lo = sum over them of min_k (d_jk + p_k) rounded down,
+// part_hi = sum of d(j, a_j) rounded up (0 for an assignment outside [0, n); the final kernel then reports no permutation).
+// A warp holds 8 bidders, its lanes split the objects, staged through shared memory 2048 at a time.  The fp64 square root is
+// taken only when the pair can lower the running minimum m: it cannot if p_k >= m or s >= t^2 with t = m - p_k rounded up
+// (then sqrt(s) >= t and d + p_k >= m), and a skipped pair leaves the minimum unchanged.
+__global__ void __launch_bounds__(kBoundThreads) emd_bound_rows_kernel(const float *__restrict__ xyz1, const float *__restrict__ xyz2,
+                                                                       const int *__restrict__ assignment, const float *__restrict__ price,
+                                                                       int n, double *__restrict__ part_lo, double *__restrict__ part_hi) {
+    __shared__ float4 obj[kBoundTile];
+    __shared__ double row_lo[kBoundRows], row_hi[kBoundRows];
+    const int cloud = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const size_t cb = (size_t)cloud * n;
+    const float *x1 = xyz1 + cb * 3, *x2 = xyz2 + cb * 3;
+    const int row0 = blockIdx.x * kBoundRows + warp * kBoundRowsPerLane;
+    float bx[kBoundRowsPerLane], by[kBoundRowsPerLane], bz[kBoundRowsPerLane];
+    double mn[kBoundRowsPerLane];
+#pragma unroll
+    for (int r = 0; r < kBoundRowsPerLane; ++r) {
+        const int j = min(row0 + r, n - 1);   // rows past the end repeat the last one and are not summed
+        bx[r] = x1[j * 3 + 0]; by[r] = x1[j * 3 + 1]; bz[r] = x1[j * 3 + 2];
+        mn[r] = __longlong_as_double(0x7ff0000000000000LL);   // +inf
+    }
+    for (int k0 = 0; k0 < n; k0 += kBoundTile) {
+        const int cnt = min(kBoundTile, n - k0);
+        __syncthreads();
+        for (int i = tid; i < cnt; i += kBoundThreads) {
+            const int k = k0 + i;
+            obj[i] = make_float4(x2[k * 3 + 0], x2[k * 3 + 1], x2[k * 3 + 2], price ? price[cb + k] : 0.f);
+        }
+        __syncthreads();
+        for (int i = lane; i < cnt; i += 32) {
+            const float4 o = obj[i];
+            const double p = (double)o.w;
+#pragma unroll
+            for (int r = 0; r < kBoundRowsPerLane; ++r) {
+                const double s = sqdist_rd(bx[r], by[r], bz[r], o.x, o.y, o.z);
+                const double t = __dsub_ru(mn[r], p);
+                if (t > 0.0 && s < __dmul_ru(t, t)) mn[r] = fmin(mn[r], __dadd_rd(__dsqrt_rd(s), p));
+            }
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < kBoundRowsPerLane; ++r) {
+        double m = mn[r];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) m = fmin(m, __shfl_xor_sync(0xffffffffu, m, o));   // exact: min is order-free
+        if (lane == r) row_lo[warp * kBoundRowsPerLane + r] = m;
+    }
+    if (lane < kBoundRowsPerLane) {
+        const int j = row0 + lane;
+        double hi = 0.0;
+        if (j < n) {
+            const int a = assignment[cb + j];
+            if (a >= 0 && a < n) hi = __dsqrt_ru(sqdist_ru(x1[j * 3 + 0], x1[j * 3 + 1], x1[j * 3 + 2], x2[a * 3 + 0], x2[a * 3 + 1], x2[a * 3 + 2]));
+        }
+        row_hi[warp * kBoundRowsPerLane + lane] = hi;
+    }
+    __syncthreads();
+    if (tid == 0) {
+        double lo = 0.0, hi = 0.0;
+        const int rows = min(kBoundRows, n - (int)blockIdx.x * kBoundRows);
+        for (int r = 0; r < rows; ++r) { lo = __dadd_rd(lo, row_lo[r]); hi = __dadd_ru(hi, row_hi[r]); }
+        part_lo[(size_t)cloud * gridDim.x + blockIdx.x] = lo;
+        part_hi[(size_t)cloud * gridDim.x + blockIdx.x] = hi;
+    }
+}
+
+// One CTA per cloud: permutation check (a bitmap of the objects in shared memory), sum_k p_k rounded up (strided partial sums,
+// then a fixed tree), the partial sums of the rows kernel in CTA order, and the per-point means.
+constexpr int kBoundFinalThreads = 1024;
+__global__ void __launch_bounds__(kBoundFinalThreads) emd_bound_final_kernel(const int *__restrict__ assignment, const float *__restrict__ price,
+                                                                             int n, int nblk, const double *__restrict__ part_lo,
+                                                                             const double *__restrict__ part_hi, double *__restrict__ bounds,
+                                                                             int *__restrict__ status) {
+    extern __shared__ unsigned int seen[];
+    __shared__ double red[kBoundFinalThreads];
+    const int cloud = blockIdx.x, tid = threadIdx.x;
+    const size_t cb = (size_t)cloud * n;
+    const int words = (n + 31) >> 5;
+    for (int w = tid; w < words; w += kBoundFinalThreads) seen[w] = 0u;
+    __syncthreads();
+    int bad = 0;
+    double ps = 0.0;
+    for (int j = tid; j < n; j += kBoundFinalThreads) {
+        const int o = assignment[cb + j];
+        if (o < 0 || o >= n) {
+            bad = 1;
+        } else {
+            const unsigned int bit = 1u << (o & 31);
+            if (atomicOr(seen + (o >> 5), bit) & bit) bad = 1;   // object taken twice
+        }
+        if (price) ps = __dadd_ru(ps, (double)price[cb + j]);
+    }
+    red[tid] = ps;
+    bad = __syncthreads_or(bad);
+    for (int s = kBoundFinalThreads / 2; s > 0; s >>= 1) {
+        if (tid < s) red[tid] = __dadd_ru(red[tid], red[tid + s]);
+        __syncthreads();
+    }
+    if (tid == 0) {
+        double lo = 0.0, hi = 0.0;
+        for (int i = 0; i < nblk; ++i) {
+            lo = __dadd_rd(lo, part_lo[(size_t)cloud * nblk + i]);
+            hi = __dadd_ru(hi, part_hi[(size_t)cloud * nblk + i]);
+        }
+        bounds[2 * (size_t)cloud + 0] = __ddiv_rd(__dsub_rd(lo, red[0]), (double)n);
+        bounds[2 * (size_t)cloud + 1] = bad ? __longlong_as_double(0x7ff8000000000000LL) : __ddiv_ru(hi, (double)n);
+        status[cloud] = bad ? 0 : 1;
+    }
+}
+
 static size_t emd_smem_bytes(int n, int S) {
     const int ns = n / S;
     return sizeof(float) * (size_t)(4 * n) + sizeof(float) * (size_t)(7 * ns) + sizeof(float) * (32 * 3 + 8 + 4);
@@ -1141,4 +1275,30 @@ cudaError_t psd_launch_emd_backward(const float *xyz1, const float *xyz2, float 
     else if (mode == 1) emd_grad_kernel<true, false><<<blocks, 256, 0, stream>>>(total, n, b, xyz1, xyz2, graddist, nullptr, idx, gradxyz);
     else emd_grad_kernel<true, true><<<blocks, 256, 0, stream>>>(total, n, b, xyz1, xyz2, graddist, upstream, idx, gradxyz);
     return cudaGetLastError();
+}
+
+int psd_emd_bound_max_points() { return 1 << 20; }   // the permutation bitmap of a cloud (n / 8 bytes) sits in shared memory
+
+// bounds[B, 2] (lower, upper per point, fp64) and status[B] of (assignment, price); price may be NULL (all zero).  Two launches
+// and a stream-ordered scratch of 2 B ceil(n / 64) doubles; nothing synchronises the host (capturable in a CUDA graph).
+cudaError_t psd_launch_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const int *assignment, const float *price,
+                                      double *bounds, int *status, cudaStream_t stream) {
+    if (b <= 0 || n <= 0) return cudaSuccess;
+    const int nblk = (n + kBoundRows - 1) / kBoundRows;
+    const size_t smem = sizeof(unsigned int) * (size_t)((n + 31) / 32);
+    cudaError_t e = cudaFuncSetAttribute(emd_bound_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    double *part = nullptr;
+    e = cudaMallocAsync(reinterpret_cast<void **>(&part), sizeof(double) * 2 * (size_t)b * nblk, stream);
+    if (e != cudaSuccess) return e;
+    double *part_lo = part, *part_hi = part + (size_t)b * nblk;
+    emd_bound_rows_kernel<<<dim3((unsigned int)nblk, (unsigned int)b), kBoundThreads, 0, stream>>>(xyz1, xyz2, assignment, price, n,
+                                                                                                 part_lo, part_hi);
+    e = cudaGetLastError();
+    if (e == cudaSuccess) {
+        emd_bound_final_kernel<<<b, kBoundFinalThreads, smem, stream>>>(assignment, price, n, nblk, part_lo, part_hi, bounds, status);
+        e = cudaGetLastError();
+    }
+    const cudaError_t e2 = cudaFreeAsync(part, stream);
+    return e != cudaSuccess ? e : e2;
 }

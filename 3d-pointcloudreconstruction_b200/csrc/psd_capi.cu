@@ -44,6 +44,9 @@ cudaError_t psd_launch_emd_forward(const float *xyz1, const float *xyz2, int b, 
 cudaError_t psd_launch_emd_mean_loss(const float *sums, int b, int n, float *out, cudaStream_t stream);
 cudaError_t psd_launch_emd_backward(const float *xyz1, const float *xyz2, float *gradxyz, const float *graddist,
                                     const int *idx, int b, int n, int mode, const float *upstream, cudaStream_t stream);
+cudaError_t psd_launch_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const int *assignment, const float *price,
+                                      double *bounds, int *status, cudaStream_t stream);
+int psd_emd_bound_max_points();
 
 static thread_local char g_err[512] = "";
 
@@ -192,6 +195,68 @@ int psd_emd_backward_ex(const float *xyz1, const float *xyz2, float *gradxyz, co
                         int b, int n, int overwrite, void *stream) {
     return finish("psd_emd_backward_ex",
                   psd_launch_emd_backward(xyz1, xyz2, gradxyz, graddist, idx, b, n, overwrite ? 1 : 0, nullptr, (cudaStream_t)stream));
+}
+
+// Certified EMD: epsilon-scaling phases of the unchanged auction kernel, then the dual-bound certificate.  Every phase starts
+// from assignment = -1 and the previous phase's prices (the kernel reads and writes back the caller's price buffer when
+// fresh = 0; NULL assignment_inv / max_increments start at -1 / 0 as in the reference's initial state).  Phase i runs
+// eps = max(eps_start / scale^i, eps_end) (in double, rounded to float), the last one exactly eps_end.  No host synchronisation.
+static const int kEmdMaxPhases = 64;
+
+static int emd_certified_common(const char *what, const float *xyz1, const float *xyz2, int b, int n, float eps_start,
+                                float eps_end, float scale, int max_iters_per_phase, float *dist, int *assignment, float *price,
+                                double *bounds, int *status, int force_cluster, void *stream_) {
+    char msg[256];
+    if (b < 0 || b > 512) { snprintf(msg, sizeof(msg), "%s: the batch size must be in [0, 512]", what); psd_set_error_msg(msg); return -1; }
+    if (n <= 0 || n % 1024 != 0) { snprintf(msg, sizeof(msg), "%s: the size of the point clouds must be a positive multiple of 1024", what); psd_set_error_msg(msg); return -1; }
+    if (!(eps_end >= 1e-5f)) { snprintf(msg, sizeof(msg), "%s: eps_end must be >= 1e-5 (the auction's fp32 prices and +-1e-6 winner window make a smaller eps meaningless)", what); psd_set_error_msg(msg); return -1; }
+    if (!(eps_end <= eps_start)) { snprintf(msg, sizeof(msg), "%s: eps_end must not exceed eps_start", what); psd_set_error_msg(msg); return -1; }
+    if (!(scale > 1.0f)) { snprintf(msg, sizeof(msg), "%s: scale must be > 1", what); psd_set_error_msg(msg); return -1; }
+    if (max_iters_per_phase < 1) { snprintf(msg, sizeof(msg), "%s: max_iters_per_phase must be >= 1", what); psd_set_error_msg(msg); return -1; }
+    int phases = 1;
+    for (double e = eps_start; e > (double)eps_end && phases <= kEmdMaxPhases; e /= (double)scale) ++phases;
+    if (phases > kEmdMaxPhases) { snprintf(msg, sizeof(msg), "%s: more than %d phases (scale too close to 1)", what, kEmdMaxPhases); psd_set_error_msg(msg); return -1; }
+    if (b == 0) return 1;
+    cudaStream_t stream = (cudaStream_t)stream_;
+    const size_t cells = (size_t)b * n;
+    cudaError_t e = cudaMemsetAsync(price, 0, sizeof(float) * cells, stream);
+    double e_cur = eps_start;
+    for (int ph = 0; ph < phases && e == cudaSuccess; ++ph, e_cur /= (double)scale) {
+        const float eps = ph == phases - 1 ? eps_end : (float)e_cur;
+        e = cudaMemsetAsync(assignment, 0xff, sizeof(int) * cells, stream);   // every point unassigned (-1)
+        int unsupported = 0;
+        if (e == cudaSuccess)
+            e = psd_launch_emd_forward(xyz1, xyz2, b, n, dist, assignment, price, nullptr, nullptr, nullptr, nullptr, eps,
+                                       max_iters_per_phase, force_cluster, 0, nullptr, stream, &unsupported);
+        if (unsupported) { psd_set_error_msg(kEmdShapeMsg); return 0; }
+    }
+    if (e == cudaSuccess) e = psd_launch_emd_dual_bound(xyz1, xyz2, b, n, assignment, price, bounds, status, stream);
+    return finish(what, e);
+}
+
+int psd_emd_certified(const float *xyz1, const float *xyz2, int b, int n, float eps_start, float eps_end, float scale,
+                      int max_iters_per_phase, float *dist, int *assignment, float *price, double *bounds, int *status,
+                      void *stream) {
+    return emd_certified_common("psd_emd_certified", xyz1, xyz2, b, n, eps_start, eps_end, scale, max_iters_per_phase, dist,
+                                assignment, price, bounds, status, 0, stream);
+}
+
+// test hook: the same with the cluster size of every phase forced as in psd_emd_forward_cluster
+int psd_emd_certified_cluster(const float *xyz1, const float *xyz2, int b, int n, float eps_start, float eps_end, float scale,
+                              int max_iters_per_phase, float *dist, int *assignment, float *price, double *bounds, int *status,
+                              int cluster_size, void *stream) {
+    return emd_certified_common("psd_emd_certified_cluster", xyz1, xyz2, b, n, eps_start, eps_end, scale, max_iters_per_phase,
+                                dist, assignment, price, bounds, status, cluster_size, stream);
+}
+
+int psd_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const int *assignment, const float *price,
+                       double *bounds, int *status, void *stream) {
+    if (b < 0 || b > 65535 || n < 1 || n > psd_emd_bound_max_points()) {
+        psd_set_error_msg("psd_emd_dual_bound: b in [0, 65535] and n in [1, 2^20] required");
+        return -1;
+    }
+    return finish("psd_emd_dual_bound",
+                  psd_launch_emd_dual_bound(xyz1, xyz2, b, n, assignment, price, bounds, status, (cudaStream_t)stream));
 }
 
 int psd_emd_mean_loss_forward(const float *xyz1, const float *xyz2, int b, int n, float *dist, int *assignment, float eps,

@@ -1,5 +1,6 @@
 """Evaluation-metric glue of the hot path (mirrors utils/metrics.py): EMD (eps=0.005, iters=50) and Chamfer
-distance, both x100, plus the registry / best-value comparison the eval drivers use."""
+distance, both x100, plus the registry / best-value comparison the eval drivers use.  certified_emd_distance is an
+extra: the EMD of a true matching with a bound on its distance from the optimum."""
 import logging
 
 import torch
@@ -10,6 +11,19 @@ try:
 except ImportError:
     from dist_chamfer_3D import chamfer_3DDist
     import emd_module as emd_func
+
+
+def certified_emd_distance(pred, gt, eps_end=1e-4):
+    """EMD of pred against gt with a certificate, x100 like Metrics._get_emd_distance: returns (value, gap).
+
+    value = sqrt(dist).mean(1).mean() * 100 over the epsilon-scaled auction's matching (emd_module.emd_certified);
+    gap = mean over the clouds of (upper - lower) * 100, a bound on how far value can be from the batch mean of the
+    optimal EMDs.  gap is NaN when a cloud did not end with a matching."""
+    with torch.no_grad():
+        dist, _, bounds, _ = emd_func.emd_certified(pred, gt, eps_end=eps_end)
+        value = torch.sqrt(dist).mean(1).mean().item() * 100
+        gap = (bounds[:, 1] - bounds[:, 0]).mean().item() * 100
+    return value, gap
 
 
 class Metrics(object):

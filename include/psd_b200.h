@@ -124,6 +124,42 @@ int psd_emd_backward(const float *xyz1, const float *xyz2, float *gradxyz, const
 int psd_emd_backward_ex(const float *xyz1, const float *xyz2, float *gradxyz, const float *graddist, const int *idx,
                         int b, int n, int overwrite, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Certified earth mover's distance (not part of the reference surface).
+ * ------------------------------------------------------------------------------------------- */
+
+/* Weak-duality certificate of an (assignment, prices) pair.  With d_jk = |xyz1[b,j] - xyz2[b,k]| (Euclidean, not squared):
+ *   L = sum_j min_k (d_jk + price[b,k]) - sum_k price[b,k]  <=  optimal matching cost  <=  U = sum_j d(j, assignment[b,j])
+ * where L holds for ANY prices and U whenever the assignment is a permutation.  Outputs per cloud: bounds[b] = (L / n, U / n)
+ * fp64, the unit of sqrt(dist).mean(1); status[b] = 1 (a permutation, both bounds valid) or 0 (not a permutation: the lower
+ * bound is still valid, the upper one is NaN).  Every term is rounded towards its bound (fp64 directed rounding) and the sums
+ * run in a fixed order, so the bounds are rigorous for the fp32 inputs and reproducible bit for bit.  price may be NULL (all
+ * zero).  Any n in [1, 2^20], b <= 65535; about one fp64 evaluation of every pair.  Returns 1 / 0 CUDA error / -1 argument. */
+int psd_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const int *assignment, const float *price,
+                       double *bounds, int *status, void *stream);
+
+/* The auction run to a true matching by epsilon-scaling, with its certificate.  Phases with eps = eps_start, eps_start / scale,
+ * ... (computed in double, rounded to float) down to exactly eps_end, each one the auction of psd_emd_forward started from
+ * assignment = -1 and the PREVIOUS phase's prices, run until every point is assigned or max_iters_per_phase iterations (a phase
+ * that runs out of iterations ends with the auction's forced assignment, which the certificate reports as status 0; several
+ * winners of one object then add to its price in the same iteration, as in the reference, so such a result is not
+ * reproducible bit for bit, while its certificate stays valid).  Then
+ * psd_emd_dual_bound on the final (assignment, price).  Outputs: dist [B, n] (squared, as psd_emd_forward), assignment [B, n],
+ * price [B, n] (final prices), bounds [B, 2], status [B].  U - L <= eps_end per point is what epsilon-complementary slackness
+ * gives; the certificate measures it instead of assuming it.  Everything is enqueued on `stream` with no host
+ * synchronisation (a call can be captured in a CUDA graph); one launch per phase plus two for the certificate.
+ * Limits of psd_emd_forward (b <= 512, n % 1024 == 0, coordinates in [0, 1]); -1 also for eps_end < 1e-5 (the kernel's fp32
+ * prices and +-1e-6 winner window make a smaller eps meaningless), eps_end > eps_start, scale <= 1, max_iters_per_phase < 1 and
+ * more than 64 phases. */
+int psd_emd_certified(const float *xyz1, const float *xyz2, int b, int n, float eps_start, float eps_end, float scale,
+                      int max_iters_per_phase, float *dist, int *assignment, float *price, double *bounds, int *status,
+                      void *stream);
+/* Test hook: psd_emd_certified with the cluster size of every phase forced as in psd_emd_forward_cluster (negative = the
+ * global-workspace form). */
+int psd_emd_certified_cluster(const float *xyz1, const float *xyz2, int b, int n, float eps_start, float eps_end, float scale,
+                              int max_iters_per_phase, float *dist, int *assignment, float *price, double *bounds, int *status,
+                              int cluster_size, void *stream);
+
 /* Fused training loss of the EMD term: Loss.get_emd_loss (loss/loss.py:18-28) = sqrt(dist).mean(1).mean() over emdModule's
  * distances.  Forward: the auction kernel adds sum_j sqrt(dist[b, j]) to sums_zeroed[b] (zero-filled by the caller) in its
  * CalcDist tail and a one-warp kernel reduces them to the scalar *loss (device); dist / assignment are still written.
