@@ -1043,7 +1043,9 @@ __global__ void emd_mean_loss_kernel(const float *__restrict__ sums, int b, floa
 // is the cost of a feasible matching, so L <= optimum <= U.  Nothing about the auction is assumed.  Every quantity is
 // rounded towards its bound: d_jk + p_k downwards for L (|dx| rounded down, squares and sums of squares rounded down,
 // __dsqrt_rd), sum_k p_k upwards; d(j, a_j) upwards for U.  The sums run in a fixed order (no float atomics): the bounds are
-// reproducible bit for bit.
+// reproducible bit for bit.  A cloud with a NaN or infinite coordinate has no certificate: both bounds NaN, status 0 (the
+// final kernel checks; fmaxf / fminf in absdiff_* would otherwise read a NaN difference as 0).  A NaN price makes sum_k p_k
+// and so the lower bound NaN; the upper bound does not involve prices.
 constexpr int kBoundThreads = 256;
 constexpr int kBoundRowsPerLane = 8;                                   // bidders per warp; every lane carries all of them
 constexpr int kBoundRows = (kBoundThreads / 32) * kBoundRowsPerLane;   // 64 bidders per CTA
@@ -1128,10 +1130,12 @@ __global__ void __launch_bounds__(kBoundThreads) emd_bound_rows_kernel(const flo
     }
 }
 
-// One CTA per cloud: permutation check (a bitmap of the objects in shared memory), sum_k p_k rounded up (strided partial sums,
-// then a fixed tree), the partial sums of the rows kernel in CTA order, and the per-point means.
+// One CTA per cloud: permutation check (a bitmap of the objects in shared memory), finiteness of both clouds' coordinates,
+// sum_k p_k rounded up (strided partial sums, then a fixed tree), the partial sums of the rows kernel in CTA order, and the
+// per-point means.
 constexpr int kBoundFinalThreads = 1024;
-__global__ void __launch_bounds__(kBoundFinalThreads) emd_bound_final_kernel(const int *__restrict__ assignment, const float *__restrict__ price,
+__global__ void __launch_bounds__(kBoundFinalThreads) emd_bound_final_kernel(const float *__restrict__ xyz1, const float *__restrict__ xyz2,
+                                                                             const int *__restrict__ assignment, const float *__restrict__ price,
                                                                              int n, int nblk, const double *__restrict__ part_lo,
                                                                              const double *__restrict__ part_hi, double *__restrict__ bounds,
                                                                              int *__restrict__ status) {
@@ -1142,9 +1146,11 @@ __global__ void __launch_bounds__(kBoundFinalThreads) emd_bound_final_kernel(con
     const int words = (n + 31) >> 5;
     for (int w = tid; w < words; w += kBoundFinalThreads) seen[w] = 0u;
     __syncthreads();
-    int bad = 0;
+    int bad = 0, nonfinite = 0;
     double ps = 0.0;
     for (int j = tid; j < n; j += kBoundFinalThreads) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) nonfinite |= !isfinite(xyz1[(cb + j) * 3 + c]) || !isfinite(xyz2[(cb + j) * 3 + c]);
         const int o = assignment[cb + j];
         if (o < 0 || o >= n) {
             bad = 1;
@@ -1156,6 +1162,7 @@ __global__ void __launch_bounds__(kBoundFinalThreads) emd_bound_final_kernel(con
     }
     red[tid] = ps;
     bad = __syncthreads_or(bad);
+    nonfinite = __syncthreads_or(nonfinite);
     for (int s = kBoundFinalThreads / 2; s > 0; s >>= 1) {
         if (tid < s) red[tid] = __dadd_ru(red[tid], red[tid + s]);
         __syncthreads();
@@ -1166,9 +1173,10 @@ __global__ void __launch_bounds__(kBoundFinalThreads) emd_bound_final_kernel(con
             lo = __dadd_rd(lo, part_lo[(size_t)cloud * nblk + i]);
             hi = __dadd_ru(hi, part_hi[(size_t)cloud * nblk + i]);
         }
-        bounds[2 * (size_t)cloud + 0] = __ddiv_rd(__dsub_rd(lo, red[0]), (double)n);
-        bounds[2 * (size_t)cloud + 1] = bad ? __longlong_as_double(0x7ff8000000000000LL) : __ddiv_ru(hi, (double)n);
-        status[cloud] = bad ? 0 : 1;
+        const double nan = __longlong_as_double(0x7ff8000000000000LL);
+        bounds[2 * (size_t)cloud + 0] = nonfinite ? nan : __ddiv_rd(__dsub_rd(lo, red[0]), (double)n);
+        bounds[2 * (size_t)cloud + 1] = bad || nonfinite ? nan : __ddiv_ru(hi, (double)n);
+        status[cloud] = bad || nonfinite ? 0 : 1;
     }
 }
 
@@ -1296,7 +1304,8 @@ cudaError_t psd_launch_emd_dual_bound(const float *xyz1, const float *xyz2, int 
                                                                                                  part_lo, part_hi);
     e = cudaGetLastError();
     if (e == cudaSuccess) {
-        emd_bound_final_kernel<<<b, kBoundFinalThreads, smem, stream>>>(assignment, price, n, nblk, part_lo, part_hi, bounds, status);
+        emd_bound_final_kernel<<<b, kBoundFinalThreads, smem, stream>>>(xyz1, xyz2, assignment, price, n, nblk, part_lo, part_hi,
+                                                                          bounds, status);
         e = cudaGetLastError();
     }
     const cudaError_t e2 = cudaFreeAsync(part, stream);

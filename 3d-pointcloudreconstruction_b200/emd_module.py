@@ -129,5 +129,6 @@ def emd_certified(xyz1, xyz2, eps_end=1e-4, eps_start=0.05, scale=4.0, max_iters
       * bounds [B, 2] fp64, (lower, upper) on the optimal EMD per point, the unit of ``sqrt(dist).mean(1)``:
         lower <= true EMD <= upper, with upper - lower <= eps_end in practice;
       * status [B] int32, 1 = permutation (both bounds valid), 0 = a phase ran out of ``max_iters_per_phase`` and the result
-        is not a matching (lower bound still valid, upper is NaN)."""
+        is not a matching (lower bound still valid, upper is NaN), or a cloud has a NaN or infinite coordinate (no
+        certificate: both bounds NaN)."""
     return emdCertifiedFunction.apply(xyz1, xyz2, float(eps_end), float(eps_start), float(scale), int(max_iters_per_phase))

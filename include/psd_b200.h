@@ -134,7 +134,9 @@ int psd_emd_backward_ex(const float *xyz1, const float *xyz2, float *gradxyz, co
  * fp64, the unit of sqrt(dist).mean(1); status[b] = 1 (a permutation, both bounds valid) or 0 (not a permutation: the lower
  * bound is still valid, the upper one is NaN).  Every term is rounded towards its bound (fp64 directed rounding) and the sums
  * run in a fixed order, so the bounds are rigorous for the fp32 inputs and reproducible bit for bit.  price may be NULL (all
- * zero).  Any n in [1, 2^20], b <= 65535; about one fp64 evaluation of every pair.  Returns 1 / 0 CUDA error / -1 argument. */
+ * zero).  A cloud with a NaN or infinite coordinate in xyz1 or xyz2 has no certificate: both bounds NaN, status 0.  A NaN
+ * price makes the lower bound NaN (the upper bound and status do not depend on prices).  Any n in [1, 2^20], b <= 65535;
+ * about one fp64 evaluation of every pair.  Returns 1 / 0 CUDA error / -1 argument. */
 int psd_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const int *assignment, const float *price,
                        double *bounds, int *status, void *stream);
 
