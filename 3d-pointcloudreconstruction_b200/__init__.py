@@ -20,9 +20,10 @@ from .emd_module import emdFunction, emdModule, emd_certified
 from .fscore import fscore, chamfer_fscore_fused
 from .loss import Loss, chamfer_loss_step_host, ChamferLossPipeline
 from .metrics import Metrics, certified_emd_distance
+from .sinkhorn import sinkhornFunction, sinkhorn_divergence
 
 __all__ = [
     "chamfer_3D", "emd", "proj_loss", "icp", "projection", "utils", "loss_", "chamfer_3DDist", "chamfer_3DFunction", "emdFunction", "emdModule",
     "fscore", "chamfer_fscore_fused", "Loss", "chamfer_loss_step_host", "ChamferLossPipeline", "Metrics",
-    "emd_certified", "certified_emd_distance",
+    "emd_certified", "certified_emd_distance", "sinkhornFunction", "sinkhorn_divergence",
 ]

@@ -39,6 +39,8 @@ _SIGNATURES = {
     "psd_emd_certified_cluster": [_vp, _vp, _ci, _ci, _cf, _cf, _cf, _ci, _vp, _vp, _vp, _vp, _vp, _ci, _vp],
     "psd_emd_mean_loss_forward": [_vp, _vp, _ci, _ci, _vp, _vp, _cf, _ci, _vp, _vp, _vp],
     "psd_emd_mean_loss_backward": [_vp, _vp, _vp, _vp, _vp, _vp, _ci, _ci, _vp],
+    "psd_sinkhorn_divergence": [_vp, _vp, _ci, _ci, _ci, _cf, _cf, _vp, _vp, _vp, _vp, _vp, _vp],
+    "psd_sinkhorn_divergence_cluster": [_vp, _vp, _ci, _ci, _ci, _cf, _cf, _vp, _vp, _vp, _vp, _vp, _ci, _vp],
     "psd_chamfer_forward_host": [_vp, _vp, _ci, _ci, _ci, _vp, _vp, _vp, _vp, _vp],
     "psd_fp32_fma_peak": [_cf, ctypes.POINTER(_cf), _vp],
     "psd_chamfer_stats": [ctypes.POINTER(ctypes.c_longlong), _ci],

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libpsd_b200.so")
-SOURCES = ["chamfer.cu", "chamfer_nn_tc.cu", "emd.cu", "proj.cu", "icp.cu", "fps.cu", "splat.cu", "psd_capi.cu"]
+SOURCES = ["chamfer.cu", "chamfer_nn_tc.cu", "emd.cu", "proj.cu", "icp.cu", "fps.cu", "splat.cu", "sinkhorn.cu", "psd_capi.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

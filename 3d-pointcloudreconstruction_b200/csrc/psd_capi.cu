@@ -1,4 +1,5 @@
 // psd_capi.cu -- extern "C" surface of libpsd_b200.so (declared in include/psd_b200.h).
+#include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -47,6 +48,9 @@ cudaError_t psd_launch_emd_backward(const float *xyz1, const float *xyz2, float 
 cudaError_t psd_launch_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const int *assignment, const float *price,
                                       double *bounds, int *status, cudaStream_t stream);
 int psd_emd_bound_max_points();
+cudaError_t psd_launch_sinkhorn(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
+                                float *grad_x, float *grad_y, float *potentials, int *rounds, int force_cluster,
+                                cudaStream_t stream);
 
 static thread_local char g_err[512] = "";
 
@@ -257,6 +261,37 @@ int psd_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const
     }
     return finish("psd_emd_dual_bound",
                   psd_launch_emd_dual_bound(xyz1, xyz2, b, n, assignment, price, bounds, status, (cudaStream_t)stream));
+}
+
+static int sinkhorn_common(const char *what, const float *x, const float *y, int b, int n, int m, float blur, float scaling,
+                           float *loss, float *grad_x, float *grad_y, float *potentials, int *rounds, int force_cluster,
+                           void *stream) {
+    char msg[256];
+    const char *bad = nullptr;
+    if (b < 0 || b > 65535) bad = "the batch size must be in [0, 65535]";
+    else if (n < 1 || n > (1 << 20) || m < 1 || m > (1 << 20)) bad = "the cloud sizes n and m must be in [1, 2^20]";
+    else if (!(blur > 0.f) || !isfinite(blur)) bad = "blur must be finite and > 0";
+    else if (!(scaling > 0.f && scaling < 1.f)) bad = "scaling must be in (0, 1)";
+    else if (loss == nullptr) bad = "loss must not be NULL";
+    else if (force_cluster != 0 && force_cluster != 1 && force_cluster != 2 && force_cluster != 4 && force_cluster != 8)
+        bad = "cluster_size must be 1, 2, 4 or 8";
+    if (bad) { snprintf(msg, sizeof(msg), "%s: %s", what, bad); psd_set_error_msg(msg); return -1; }
+    if (b == 0) return 1;
+    return finish(what, psd_launch_sinkhorn(x, y, b, n, m, blur, scaling, loss, grad_x, grad_y, potentials, rounds, force_cluster,
+                                            (cudaStream_t)stream));
+}
+
+int psd_sinkhorn_divergence(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
+                            float *grad_x, float *grad_y, float *potentials, int *rounds, void *stream) {
+    return sinkhorn_common("psd_sinkhorn_divergence", x, y, b, n, m, blur, scaling, loss, grad_x, grad_y, potentials, rounds, 0,
+                           stream);
+}
+
+int psd_sinkhorn_divergence_cluster(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
+                                    float *grad_x, float *grad_y, float *potentials, int *rounds, int cluster_size, void *stream) {
+    if (cluster_size == 0) cluster_size = -1;   // 0 selects automatically inside; the hook forces a size
+    return sinkhorn_common("psd_sinkhorn_divergence_cluster", x, y, b, n, m, blur, scaling, loss, grad_x, grad_y, potentials,
+                           rounds, cluster_size, stream);
 }
 
 int psd_emd_mean_loss_forward(const float *xyz1, const float *xyz2, int b, int n, float *dist, int *assignment, float eps,

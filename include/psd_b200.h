@@ -173,6 +173,22 @@ int psd_emd_mean_loss_forward(const float *xyz1, const float *xyz2, int b, int n
 int psd_emd_mean_loss_backward(const float *xyz1, const float *xyz2, float *gradxyz1, const float *dist, const int *assignment,
                                const float *upstream, int b, int n, void *stream);
 
+/* Debiased Sinkhorn divergence per cloud pair (geomloss SamplesLoss("sinkhorn", p=2, blur, scaling, debias=True), uniform
+ * weights, cost |u - v|^2 / 2), for clouds x [b, n, 3] and y [b, m, 3] of any sizes, anywhere in space.  The epsilon schedule
+ * runs from the squared diameter of both clouds down to blur^2 by factors scaling^2; rounds[b] (optional) receives its length,
+ * len(eps_list).  Outputs: loss[b] = S; grad_x [b, n, 3] and grad_y [b, m, 3] (each optional) dS/dx and dS/dy of geomloss's
+ * last extrapolation step; potentials [b, 2n + 2m] (optional) the final f_ba, f_aa (n each), g_ab, g_bb (m each).  A pair
+ * whose points all coincide gives S = 0, zero gradients and potentials, 0 rounds; a pair with a NaN or infinite coordinate
+ * gives NaN everywhere and 0 rounds, without affecting the other pairs.  Deterministic: no float atomics, and the result does
+ * not depend on the launch decomposition.  One launch plus a stream-ordered workspace of 2 (2n + 2m) floats per pair; no host
+ * synchronisation (capturable in a CUDA graph).  Returns 1 / 0 CUDA error / -1 argument: b outside [0, 65535], n or m
+ * outside [1, 2^20], blur not finite and > 0, scaling outside (0, 1), loss NULL.  b = 0 does nothing and returns 1. */
+int psd_sinkhorn_divergence(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
+                            float *grad_x, float *grad_y, float *potentials, int *rounds, void *stream);
+/* Test hook: the same with the cluster size (CTAs per cloud pair) forced to 1, 2, 4 or 8 (-1 for another value). */
+int psd_sinkhorn_divergence_cluster(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
+                                    float *grad_x, float *grad_y, float *potentials, int *rounds, int cluster_size, void *stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Fused training loss of the hot path's caller: Loss.get_chamfer_loss (loss/loss.py:30-37) =
  * mean(dist1) + mean(dist2) over chamfer_3DDist's outputs.  Forward: the NN kernel accumulates per-cloud sums in its
