@@ -29,6 +29,7 @@ constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kHalfLog2e = 0.7213475204444817f;
 constexpr float kLn2 = 0.6931471805599453f;
 constexpr long long kSkMaxLoopEps = 1 << 30;
+constexpr float kSkMinEps = 0x1p-128f;  // the least eps for which kHalfLog2e / eps is finite, to a power of 2
 
 struct SkParams {
     const float *x, *y;
@@ -52,12 +53,16 @@ struct Lse {
 };
 
 // epsilon of round t (0 = init at eps_list[0], 1..K = eps_list[t-1], K + 1 = extrapolation at blur^2), K = L + 2: computed in
-// double, rounded to fp32
+// double, rounded to fp32, and raised to at least kSkMinEps.  Below it kk = kHalfLog2e / eps overflows and a query's own
+// target gives fma(-0, inf, h) = NaN; only D < 5.4e-20 (eps_list[0] = D^2) or blur < 5.4e-20 reach it.  For a tiny D the
+// raised rounds are those at D^2, whose potentials (of order D^2) vanish against blur^2 in the later rounds' h.
 __device__ __forceinline__ float eps_of_round(int t, long long L, double D, double lnD2, double lnS2, float blur) {
     const long long i = t == 0 ? 0 : t - 1;             // index into eps_list
-    if (i == 0) return (float)(D * D);
-    if (i <= L) return (float)exp(lnD2 + (double)(i - 1) * lnS2);
-    return (float)((double)blur * (double)blur);
+    double e;
+    if (i == 0) e = D * D;
+    else if (i <= L) e = exp(lnD2 + (double)(i - 1) * lnS2);
+    else e = (double)blur * (double)blur;
+    return fmaxf((float)e, kSkMinEps);
 }
 
 template <bool GRAD>

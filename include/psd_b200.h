@@ -175,8 +175,9 @@ int psd_emd_mean_loss_backward(const float *xyz1, const float *xyz2, float *grad
 
 /* Debiased Sinkhorn divergence per cloud pair (geomloss SamplesLoss("sinkhorn", p=2, blur, scaling, debias=True), uniform
  * weights, cost |u - v|^2 / 2), for clouds x [b, n, 3] and y [b, m, 3] of any sizes, anywhere in space.  The epsilon schedule
- * runs from the squared diameter of both clouds down to blur^2 by factors scaling^2; rounds[b] (optional) receives its length,
- * len(eps_list).  Outputs: loss[b] = S; grad_x [b, n, 3] and grad_y [b, m, 3] (each optional) dS/dx and dS/dy of geomloss's
+ * runs from the squared diameter of both clouds down to blur^2 by factors scaling^2, each value rounded to fp32 and raised to
+ * at least 2^-128 so that 1/eps stays finite (this changes only a diameter or blur below 5.4e-20); rounds[b] (optional)
+ * receives its length, len(eps_list).  Outputs: loss[b] = S; grad_x [b, n, 3] and grad_y [b, m, 3] (each optional) dS/dx and dS/dy of geomloss's
  * last extrapolation step; potentials [b, 2n + 2m] (optional) the final f_ba, f_aa (n each), g_ab, g_bb (m each).  A pair
  * whose points all coincide gives S = 0, zero gradients and potentials, 0 rounds; a pair with a NaN or infinite coordinate
  * gives NaN everywhere and 0 rounds, without affecting the other pairs.  Deterministic: no float atomics, and the result does
