@@ -48,7 +48,8 @@ cudaError_t psd_launch_emd_backward(const float *xyz1, const float *xyz2, float 
 cudaError_t psd_launch_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const int *assignment, const float *price,
                                       double *bounds, int *status, cudaStream_t stream);
 int psd_emd_bound_max_points();
-cudaError_t psd_launch_sinkhorn(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
+cudaError_t psd_launch_sinkhorn(const float *x, const float *y, int b, int n, int m, bool ragged, const int *x_len,
+                                const int *y_len, const float *x_w, const float *y_w, float blur, float scaling, float *loss,
                                 float *grad_x, float *grad_y, float *potentials, int *rounds, int force_cluster,
                                 cudaStream_t stream);
 
@@ -263,7 +264,8 @@ int psd_emd_dual_bound(const float *xyz1, const float *xyz2, int b, int n, const
                   psd_launch_emd_dual_bound(xyz1, xyz2, b, n, assignment, price, bounds, status, (cudaStream_t)stream));
 }
 
-static int sinkhorn_common(const char *what, const float *x, const float *y, int b, int n, int m, float blur, float scaling,
+static int sinkhorn_common(const char *what, const float *x, const float *y, int b, int n, int m, bool ragged,
+                           const int *x_len, const int *y_len, const float *x_w, const float *y_w, float blur, float scaling,
                            float *loss, float *grad_x, float *grad_y, float *potentials, int *rounds, int force_cluster,
                            void *stream) {
     char msg[256];
@@ -277,21 +279,37 @@ static int sinkhorn_common(const char *what, const float *x, const float *y, int
         bad = "cluster_size must be 1, 2, 4 or 8";
     if (bad) { snprintf(msg, sizeof(msg), "%s: %s", what, bad); psd_set_error_msg(msg); return -1; }
     if (b == 0) return 1;
-    return finish(what, psd_launch_sinkhorn(x, y, b, n, m, blur, scaling, loss, grad_x, grad_y, potentials, rounds, force_cluster,
-                                            (cudaStream_t)stream));
+    return finish(what, psd_launch_sinkhorn(x, y, b, n, m, ragged, x_len, y_len, x_w, y_w, blur, scaling, loss, grad_x, grad_y,
+                                            potentials, rounds, force_cluster, (cudaStream_t)stream));
 }
 
 int psd_sinkhorn_divergence(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
                             float *grad_x, float *grad_y, float *potentials, int *rounds, void *stream) {
-    return sinkhorn_common("psd_sinkhorn_divergence", x, y, b, n, m, blur, scaling, loss, grad_x, grad_y, potentials, rounds, 0,
-                           stream);
+    return sinkhorn_common("psd_sinkhorn_divergence", x, y, b, n, m, false, nullptr, nullptr, nullptr, nullptr, blur, scaling, loss,
+                           grad_x, grad_y, potentials, rounds, 0, stream);
 }
 
 int psd_sinkhorn_divergence_cluster(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
                                     float *grad_x, float *grad_y, float *potentials, int *rounds, int cluster_size, void *stream) {
     if (cluster_size == 0) cluster_size = -1;   // 0 selects automatically inside; the hook forces a size
-    return sinkhorn_common("psd_sinkhorn_divergence_cluster", x, y, b, n, m, blur, scaling, loss, grad_x, grad_y, potentials,
-                           rounds, cluster_size, stream);
+    return sinkhorn_common("psd_sinkhorn_divergence_cluster", x, y, b, n, m, false, nullptr, nullptr, nullptr, nullptr, blur,
+                           scaling, loss, grad_x, grad_y, potentials, rounds, cluster_size, stream);
+}
+
+int psd_sinkhorn_divergence_weighted(const float *x, const float *y, int b, int n, int m, const int *x_len, const int *y_len,
+                                     const float *x_w, const float *y_w, float blur, float scaling, float *loss, float *grad_x,
+                                     float *grad_y, float *potentials, int *rounds, void *stream) {
+    return sinkhorn_common("psd_sinkhorn_divergence_weighted", x, y, b, n, m, true, x_len, y_len, x_w, y_w, blur, scaling, loss,
+                           grad_x, grad_y, potentials, rounds, 0, stream);
+}
+
+int psd_sinkhorn_divergence_weighted_cluster(const float *x, const float *y, int b, int n, int m, const int *x_len,
+                                             const int *y_len, const float *x_w, const float *y_w, float blur, float scaling,
+                                             float *loss, float *grad_x, float *grad_y, float *potentials, int *rounds,
+                                             int cluster_size, void *stream) {
+    if (cluster_size == 0) cluster_size = -1;
+    return sinkhorn_common("psd_sinkhorn_divergence_weighted_cluster", x, y, b, n, m, true, x_len, y_len, x_w, y_w, blur, scaling,
+                           loss, grad_x, grad_y, potentials, rounds, cluster_size, stream);
 }
 
 int psd_emd_mean_loss_forward(const float *xyz1, const float *xyz2, int b, int n, float *dist, int *assignment, float eps,

@@ -189,6 +189,26 @@ int psd_sinkhorn_divergence(const float *x, const float *y, int b, int n, int m,
 /* Test hook: the same with the cluster size (CTAs per cloud pair) forced to 1, 2, 4 or 8 (-1 for another value). */
 int psd_sinkhorn_divergence_cluster(const float *x, const float *y, int b, int n, int m, float blur, float scaling, float *loss,
                                     float *grad_x, float *grad_y, float *potentials, int *rounds, int cluster_size, void *stream);
+/* The same for ragged and weighted batches.  x [b, n, 3] and y [b, m, 3] are padded; pair c takes part with its first
+ * x_len[c] points of x and y_len[c] points of y (device int [b]; NULL = n / m for every pair), with the point weights
+ * x_w [b, n] and y_w [b, m] (device fp32; NULL = uniform 1 / length).  Points beyond the lengths are never read.  The
+ * diameter, the schedule and every softmin use the participating points only; a weight w enters as log w in the softmins
+ * (a weight of 0 removes the point as a target), as w in the gradient row and in S = sum_i a_i (f_ba - f_aa) +
+ * sum_j b_j (g_ab - g_bb), summed in fp64.  Weights are not normalised: that they sum to 1 per side is the caller's contract,
+ * as in geomloss.  Outputs keep the padded shapes; gradient rows and potential entries beyond the lengths are 0.  A pair gets
+ * NaN loss, NaN in every gradient and potential row and 0 rounds, without affecting the others, when a coordinate is not
+ * finite, a length is outside [1, n] / [1, m], a participating weight is negative, NaN or infinite, or all participating
+ * weights of one side are 0.  Each pair gives the bits of a psd_sinkhorn_divergence call on its participating points alone
+ * when the weights are NULL.  Same argument checks and return convention as psd_sinkhorn_divergence; lengths and weights are
+ * device data and are not checked on the host. */
+int psd_sinkhorn_divergence_weighted(const float *x, const float *y, int b, int n, int m, const int *x_len, const int *y_len,
+                                     const float *x_w, const float *y_w, float blur, float scaling, float *loss, float *grad_x,
+                                     float *grad_y, float *potentials, int *rounds, void *stream);
+/* Test hook: the same with the cluster size forced as in psd_sinkhorn_divergence_cluster. */
+int psd_sinkhorn_divergence_weighted_cluster(const float *x, const float *y, int b, int n, int m, const int *x_len,
+                                             const int *y_len, const float *x_w, const float *y_w, float blur, float scaling,
+                                             float *loss, float *grad_x, float *grad_y, float *potentials, int *rounds,
+                                             int cluster_size, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Fused training loss of the hot path's caller: Loss.get_chamfer_loss (loss/loss.py:30-37) =
