@@ -15,7 +15,7 @@ from . import icp              # utils/icp.py mirror (icp, best_fit_transform, n
 from . import projection       # utils/projection.py mirror (cont_proj, apply_kernel)
 from . import utils            # utils/utils.py sampling helpers (farthest_point_sample, index_points)
 from . import loss_            # loss/loss_.py mirror (cd, distChamfer, batch_NN_loss, fscore) on the CUDA op
-from .dist_chamfer_3D import chamfer_3DDist, chamfer_3DFunction
+from .dist_chamfer_3D import chamfer_3DDist, chamfer_3DFunction, chamfer_ragged
 from .emd_module import emdFunction, emdModule, emd_certified
 from .fscore import fscore, chamfer_fscore_fused
 from .loss import Loss, chamfer_loss_step_host, ChamferLossPipeline
@@ -23,7 +23,7 @@ from .metrics import Metrics, certified_emd_distance
 from .sinkhorn import pack_clouds, sinkhornFunction, sinkhorn_divergence
 
 __all__ = [
-    "chamfer_3D", "emd", "proj_loss", "icp", "projection", "utils", "loss_", "chamfer_3DDist", "chamfer_3DFunction", "emdFunction", "emdModule",
+    "chamfer_3D", "emd", "proj_loss", "icp", "projection", "utils", "loss_", "chamfer_3DDist", "chamfer_3DFunction", "chamfer_ragged", "emdFunction", "emdModule",
     "fscore", "chamfer_fscore_fused", "Loss", "chamfer_loss_step_host", "ChamferLossPipeline", "Metrics",
     "emd_certified", "certified_emd_distance", "sinkhornFunction", "sinkhorn_divergence", "pack_clouds",
 ]

@@ -29,6 +29,9 @@ _SIGNATURES = {
     "psd_chamfer_forward_zero": [_vp, _vp, _ci, _ci, _ci, _ci, _vp, _vp, _vp, _vp, _vp, _cf, _vp, _vp, ctypes.c_longlong, _vp],
     "psd_chamfer_backward": [_vp] * 8 + [_ci, _ci, _ci, _vp],
     "psd_chamfer_backward_ex": [_vp] * 8 + [_ci, _ci, _ci, _ci, _ci, _vp],
+    "psd_chamfer_forward_ragged": [_vp, _vp, _ci, _ci, _ci, _ci, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _cf, _vp, _vp,
+                                   ctypes.c_longlong, _vp],
+    "psd_chamfer_backward_ragged": [_vp] * 10 + [_ci, _ci, _ci, _ci, _vp],
     "psd_emd_forward": [_vp, _vp, _ci, _ci, _ci] + [_vp] * 12 + [_cf, _ci, _vp],
     "psd_emd_forward_fresh": [_vp, _vp, _ci, _ci, _vp, _vp, _cf, _ci, _vp],
     "psd_emd_forward_cluster": [_vp, _vp, _ci, _ci, _vp, _vp, _vp, _vp, _cf, _ci, _ci, _vp],

@@ -39,12 +39,13 @@ struct BlockInfo {      // per block of the current flush group (shared memory)
     float cx, cy, cz;   // centre of the filter frame
     float t2max;        // max |t-c|^2 over the target cloud
     int bad;            // non-finite / huge target seen
-    int pad[3];
+    int qn, tn, inval;  // ragged launches: the pair's participating queries / targets (0 / 0 for an invalid pair); else 0
 };
 constexpr int kPerBlockBytes = kPartBytes + (int)sizeof(BlockInfo) + 3 * kQB * 4 + kQB * 4;  // + staged queries + fallback list
 
-template <int TM>
-__global__ void __launch_bounds__(kThreads, 1) chamfer_nn_kernel(const NNParams p) {
+// RAGGED: per-pair lengths (NNRaggedParams); blocks of the padded grid beyond them do no search.
+template <int TM, bool RAGGED>
+__global__ void __launch_bounds__(kThreads, 1) chamfer_nn_kernel(const std::conditional_t<RAGGED, NNRaggedParams, NNParams> p) {
     constexpr int Q = kQ, QB = kQB, C = kChunk;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float *sX = reinterpret_cast<float *>(smem_raw);               // SoA target tile: x, y, z, w = |t-c|^2
@@ -86,7 +87,8 @@ __global__ void __launch_bounds__(kThreads, 1) chamfer_nn_kernel(const NNParams 
             const int qbn = p.dir[bi.d].qblocks;
             bi.cloud = bid / qbn;
             bi.qblock = bid - bi.cloud * qbn;
-            bi.cx = bi.cy = bi.cz = 0.f; bi.t2max = 0.f; bi.bad = 0; bi.pad[0] = bi.pad[1] = bi.pad[2] = 0;
+            bi.cx = bi.cy = bi.cz = 0.f; bi.t2max = 0.f; bi.bad = 0; bi.qn = bi.tn = bi.inval = 0;
+            if constexpr (RAGGED) bi.inval = !ragged_lengths(p, bi.d, bi.cloud, bi.qn, bi.tn);
             binfo[tid] = bi;
         }
         __syncthreads();
@@ -96,7 +98,7 @@ __global__ void __launch_bounds__(kThreads, 1) chamfer_nn_kernel(const NNParams 
             const NNDirection &D = p.dir[bi.d];
             const float *__restrict__ qb = D.q + (long long)bi.cloud * D.q_bs;
             int j = D.q_begin + bi.qblock * QB + ql;
-            const int q_last = D.q_begin + D.q_count - 1;
+            const int q_last = RAGGED ? max(min(D.q_begin + D.q_count, bi.qn) - 1, 0) : D.q_begin + D.q_count - 1;
             j = j < q_last ? j : q_last;
             sq[(bl * 3 + 0) * QB + ql] = __ldg(qb + j * D.q_ps);
             sq[(bl * 3 + 1) * QB + ql] = __ldg(qb + j * D.q_ps + D.q_cs);
@@ -110,14 +112,15 @@ __global__ void __launch_bounds__(kThreads, 1) chamfer_nn_kernel(const NNParams 
         for (int bl = 0; bl < nb; ++bl) {
             const int d = binfo[bl].d, cloud = binfo[bl].cloud;
             const NNDirection &D = p.dir[d];
-            const int nt = D.nt;
+            // ragged: a block whose queries all lie beyond the pair's length (or of an invalid pair) scans nothing
+            const int nt = !RAGGED ? D.nt : (D.q_begin + binfo[bl].qblock * QB < binfo[bl].qn ? binfo[bl].tn : 0);
             const float *__restrict__ tb = D.t + (long long)cloud * D.t_bs;
             const long long tps = D.t_ps, tcs = D.t_cs;
             const int group = d * 0x40000000 + cloud;
 
             // centre of the filter's coordinate frame: mean of up to 8 evenly spaced targets.  Any value is
             // correct (results come from the exact formula); a centred frame only keeps the margin small.
-            if (group != c_group) {
+            if (group != c_group && (!RAGGED || nt > 0)) {
                 float sx = 0.f, sy = 0.f, sz = 0.f;
                 const int ns = nt < 8 ? nt : 8;
                 const int step = nt >> 3;
@@ -310,11 +313,18 @@ __global__ void __launch_bounds__(kThreads, 1) chamfer_nn_kernel(const NNParams 
             const int cloud = bi.cloud;
             const NNDirection &D = p.dir[bi.d];
             const int j = D.q_begin + bi.qblock * QB + ql;
-            const bool live = j < D.q_begin + D.q_count;
+            const bool live = j < D.q_begin + D.q_count && (!RAGGED || j < bi.qn);
             float dres = 0.f;
             bool done = false;
+            if (RAGGED && !live && j < D.q_begin + D.q_count) {
+                // rows past the pair's query length, and every row of an invalid pair: dist 0 (NaN), idx -1, counted nowhere
+                // (the NaN goes into the pair's sums)
+                dres = bi.inval ? __int_as_float(0x7fc00000) : 0.f;
+                D.dist[(long long)cloud * D.nq + j] = dres;
+                D.idx[(long long)cloud * D.nq + j] = -1;
+            }
             if (live) {
-                const int nt = D.nt;
+                const int nt = RAGGED ? bi.tn : D.nt;
                 const float *__restrict__ tb = D.t + (long long)cloud * D.t_bs;
                 const long long tps = D.t_ps, tcs = D.t_cs;
                 float b1 = kBig, b2 = kBig;
@@ -373,7 +383,7 @@ __global__ void __launch_bounds__(kThreads, 1) chamfer_nn_kernel(const NNParams 
                 }
             }
             if (p.sums != nullptr || p.fs_count != nullptr) {   // fused epilogues, one atomic per warp
-                float ws = done ? dres : 0.f;
+                float ws = (done || RAGGED) ? dres : 0.f;
                 int wc = (done && dres < p.fs_thr) ? 1 : 0;
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) {
@@ -399,7 +409,7 @@ __global__ void __launch_bounds__(kThreads, 1) chamfer_nn_kernel(const NNParams 
             const int cloud = bi.cloud;
             const NNDirection &D = p.dir[bi.d];
             const int j = D.q_begin + bi.qblock * QB + ql;
-            const int nt = D.nt;
+            const int nt = RAGGED ? bi.tn : D.nt;
             const float *__restrict__ tb = D.t + (long long)cloud * D.t_bs;
             const long long tps = D.t_ps, tcs = D.t_cs;
             const float x1 = sq[(bl * 3 + 0) * QB + ql], y1 = sq[(bl * 3 + 1) * QB + ql], z1 = sq[(bl * 3 + 2) * QB + ql];
@@ -510,6 +520,30 @@ __device__ __forceinline__ GradTerm grad_term(const GradParams &p, long long gid
     return t;
 }
 
+// ragged backward: per-pair lengths of xyz1 / xyz2 (device int [b], NULL = n / m)
+struct GradRaggedParams : GradParams {
+    const int *len1, *len2;
+};
+
+// The term of (direction, cloud, point) gid in a ragged backward: 1 = a term (grad_term); 0 = the point lies at or beyond its
+// cloud's length (nothing is read); 2 = the pair has a length outside [1, n] / [1, m] (t.own is set and t.v is NaN: the
+// point's gradient row becomes NaN, and there is no scatter term).
+__device__ __forceinline__ int grad_term_ragged(const GradRaggedParams &p, long long gid, GradTerm &t) {
+    const bool d2 = gid >= p.total1;
+    const long long e = d2 ? gid - p.total1 : gid;
+    const int na = d2 ? p.m : p.n;
+    const long long cloud = e / na;
+    const int j = (int)(e - cloud * na);
+    const int l1 = p.len1 ? __ldg(p.len1 + cloud) : p.n, l2 = p.len2 ? __ldg(p.len2 + cloud) : p.m;
+    const bool ok = l1 >= 1 && l1 <= p.n && l2 >= 1 && l2 <= p.m;
+    if (ok && j >= (d2 ? l2 : l1)) return 0;
+    if (ok) { t = grad_term(p, gid); return 1; }
+    t.d2 = d2;
+    t.own = cloud * 3 * na + j * (d2 ? p.ps2 : p.ps1);
+    t.v[0] = t.v[1] = t.v[2] = __int_as_float(0x7fc00000);
+    return 2;
+}
+
 // o[0], o[cs], o[2 cs] += (vx, vy, vz).  For the reference layout (cs == 1: three adjacent floats) the 8-byte aligned pair goes
 // out as ONE vector atomic (red.global.add.v2.f32, sm_90+): two instructions per term instead of three -- the kernel is bound by
 // the atomic issue rate of the SMs (786 k scalar atomics at config 2), not by bandwidth.  Each element is still added atomically.
@@ -560,14 +594,30 @@ __device__ __forceinline__ void grad_scatter(const GradParams &p, bool active, c
 // (A single cooperative launch with a grid-wide barrier in between was measured SLOWER on B200: 11.2 us against 9.4 us for the
 // two launches and 8.1 us for zero fill + MODE 0 at config 2, tools/grad_forms.py -- and it would have to wait for most of
 // the GPU when several steps are in flight.  The fast path is MODE 0 on buffers that the forward kernel zero-filled.)
-template <int MODE>
-__global__ void __launch_bounds__(256) chamfer_grad_kernel(const GradParams p) {
+// RAGGED (MODE 0 only): per-pair lengths (GradRaggedParams); points at or beyond them have no term.
+template <int MODE, bool RAGGED>
+__global__ void __launch_bounds__(256) chamfer_grad_kernel(const std::conditional_t<RAGGED, GradRaggedParams, GradParams> p) {
+    static_assert(!RAGGED || MODE == 0, "the ragged backward accumulates");
     constexpr bool OVERWRITE = MODE != 0;
     const long long nthreads = (long long)gridDim.x * blockDim.x;   // a multiple of 32
     const long long gid0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
     const bool active0 = gid0 < p.total;
     if (MODE == 0 && PSD_GRAD_TRIGGER_EARLY) pdl_trigger();   // the next forward launch may be scheduled as the SMs drain (it waits before its first global access)
+    if constexpr (RAGGED) {
+        for (long long base = gid0 - lane; base < p.total; base += nthreads) {   // warp-uniform trip count
+            GradTerm t;
+            t.d2 = false; t.own = 0; t.tgt = -1 - (long long)lane; t.v[0] = t.v[1] = t.v[2] = 0.f;
+            const int kind = base + lane < p.total ? grad_term_ragged(p, base + lane, t) : 0;
+            if (kind == 2) {   // invalid pair: NaN own row, then an inactive lane for the scatter
+                atomic_add3((t.d2 ? p.g2 : p.g1) + t.own, t.d2 ? p.cs2 : p.cs1, t.v[0], t.v[1], t.v[2]);
+                t.tgt = -1 - (long long)lane; t.v[0] = t.v[1] = t.v[2] = 0.f;
+            }
+            grad_scatter<false>(p, kind == 1, t, lane);
+        }
+        if (!PSD_GRAD_TRIGGER_EARLY) pdl_trigger();
+        return;
+    }
     GradTerm t0;
     t0.d2 = false; t0.own = 0; t0.tgt = -1 - (long long)lane; t0.v[0] = t0.v[1] = t0.v[2] = 0.f;
     if (active0) t0 = grad_term(p, gid0);
@@ -616,7 +666,8 @@ static std::atomic<int> g_tc_dbg_ld{0};
 static std::atomic<long long *> g_tc_prof{nullptr};
 
 bool psd_nn_tc_supported(const NNParams &p);                                               // chamfer_nn_tc.cu
-cudaError_t psd_launch_nn_tc(const NNParams &p, DeviceState *ds, cudaStream_t stream, float *dbg, int dbg_ld, long long *prof, int b);
+cudaError_t psd_launch_nn_tc(const NNParams &p, DeviceState *ds, cudaStream_t stream, float *dbg, int dbg_ld, long long *prof, int b,
+                             bool ragged, const int *len1, const int *len2);
 void psd_set_tc_prof(long long *prof) { g_tc_prof.store(prof); }
 cudaError_t psd_read_chamfer_stats_tc(unsigned long long *fallback, int reset);
 void psd_set_tc_debug(float *dbg, int ld) { g_tc_dbg_ld.store(ld); g_tc_dbg.store(dbg); }
@@ -634,7 +685,7 @@ static inline void layout_strides(int layout, int bit, int npts, long long &ps, 
 cudaError_t psd_launch_chamfer_forward(const float *xyz1, const float *xyz2, int b, int n, int m, int layout,
                                        float *dist1, float *dist2, int *idx1, int *idx2, float *sums, float fs_thr,
                                        int *fs_count, int q_begin, int q_count, cudaStream_t stream, float *zero_buf,
-                                       long long zero_floats) {
+                                       long long zero_floats, bool ragged, const int *len1, const int *len2) {
     if (zero_floats <= 0) zero_buf = nullptr;
     auto only_zero = [&]() { return zero_buf ? cudaMemsetAsync(zero_buf, 0, sizeof(float) * (size_t)zero_floats, stream) : cudaSuccess; };
     if (b <= 0 || n <= 0 || m <= 0) return only_zero();
@@ -673,8 +724,9 @@ cudaError_t psd_launch_chamfer_forward(const float *xyz1, const float *xyz2, int
     // B=32 N=M=1024; launches of < 2 units per SM are latency-bound and stay on the FFMA kernel (8.9 vs 7.5 us at B=8 N=512).
     const int variant = g_nn_variant.load();
     if ((variant == 3 || (variant == 0 && blocks >= 2LL * num_sms)) && psd_nn_tc_supported(p)) {
+        if (ragged) return psd_launch_nn_tc(p, ds, stream, nullptr, 0, nullptr, b, true, len1, len2);
         float *dbg = g_tc_dbg.exchange(nullptr);
-        return psd_launch_nn_tc(p, ds, stream, dbg, g_tc_dbg_ld.load(), g_tc_prof.load(), b);
+        return psd_launch_nn_tc(p, ds, stream, dbg, g_tc_dbg_ld.load(), g_tc_prof.load(), b, false, nullptr, nullptr);
     }
     // persistent grid: one CTA per SM, each takes a contiguous range of 128-query blocks
     const int grid = blocks < num_sms ? (int)blocks : num_sms;
@@ -692,16 +744,28 @@ cudaError_t psd_launch_chamfer_forward(const float *xyz1, const float *xyz2, int
     {
         std::lock_guard<std::mutex> lock(state_mutex());
         if (!ds->attr_nn) {
-            cudaError_t e = cudaFuncSetAttribute(chamfer_nn_kernel<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 1024);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(chamfer_nn_kernel<2048>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 1024);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(chamfer_nn_kernel<4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 1024);
+            cudaError_t e = cudaSuccess;
+            for (auto k : {chamfer_nn_kernel<1024, false>, chamfer_nn_kernel<2048, false>, chamfer_nn_kernel<4096, false>})
+                if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 1024);
+            for (auto k : {chamfer_nn_kernel<1024, true>, chamfer_nn_kernel<2048, true>, chamfer_nn_kernel<4096, true>})
+                if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 1024);
             if (e != cudaSuccess) return e;
             ds->attr_nn = true;
         }
     }
-    if (tile == 1024) chamfer_nn_kernel<1024><<<grid, kThreads, smem, stream>>>(p);
-    else if (tile == 2048) chamfer_nn_kernel<2048><<<grid, kThreads, smem, stream>>>(p);
-    else chamfer_nn_kernel<4096><<<grid, kThreads, smem, stream>>>(p);
+    if (ragged) {
+        NNRaggedParams pr;
+        static_cast<NNParams &>(pr) = p;
+        pr.qlen[0] = len1; pr.tlen[0] = len2;   // direction 0: xyz1 -> xyz2
+        pr.qlen[1] = len2; pr.tlen[1] = len1;
+        if (tile == 1024) chamfer_nn_kernel<1024, true><<<grid, kThreads, smem, stream>>>(pr);
+        else if (tile == 2048) chamfer_nn_kernel<2048, true><<<grid, kThreads, smem, stream>>>(pr);
+        else chamfer_nn_kernel<4096, true><<<grid, kThreads, smem, stream>>>(pr);
+        return cudaGetLastError();
+    }
+    if (tile == 1024) chamfer_nn_kernel<1024, false><<<grid, kThreads, smem, stream>>>(p);
+    else if (tile == 2048) chamfer_nn_kernel<2048, false><<<grid, kThreads, smem, stream>>>(p);
+    else chamfer_nn_kernel<4096, false><<<grid, kThreads, smem, stream>>>(p);
     return cudaGetLastError();
 }
 
@@ -713,7 +777,8 @@ cudaError_t psd_launch_chamfer_mean_loss(const float *sums, int b, int n, int m,
 // overwrite = 0: accumulate into caller-zeroed gradients (the reference's contract); 1: the gradients need no initialisation
 cudaError_t psd_launch_chamfer_backward(const float *xyz1, const float *xyz2, float *gradxyz1, float *gradxyz2,
                                         const float *graddist1, const float *graddist2, const int *idx1, const int *idx2,
-                                        int b, int n, int m, int layout, int overwrite, cudaStream_t stream, const float *upstream) {
+                                        int b, int n, int m, int layout, int overwrite, cudaStream_t stream, const float *upstream,
+                                        bool ragged, const int *len1, const int *len2) {
     if (b <= 0 || (n <= 0 && m <= 0)) return cudaSuccess;
     if (n <= 0 || m <= 0) {   // one cloud is empty: no pair exists, nothing to accumulate
         if (!overwrite) return cudaSuccess;
@@ -731,16 +796,23 @@ cudaError_t psd_launch_chamfer_backward(const float *xyz1, const float *xyz2, fl
     layout_strides(layout, 2, m, p.ps2, p.cs2);
     const long long blocks = (p.total + 255) / 256;
     if (blocks > 0x7fffffffLL) return cudaErrorInvalidConfiguration;
+    if (ragged) {   // (accumulate form only)
+        GradRaggedParams pr;
+        static_cast<GradParams &>(pr) = p;
+        pr.len1 = len1; pr.len2 = len2;
+        chamfer_grad_kernel<0, true><<<(unsigned int)blocks, 256, 0, stream>>>(pr);
+        return cudaGetLastError();
+    }
     if (!overwrite) {
         // A PLAIN launch: as a programmatic dependent of the forward kernel the 512 small CTAs are placed as the forward's CTAs
         // exit -- eight per SM on the first SMs to drain, none on the last ones -- and the kernel runs on half of the GPU
         // (38.9 instead of 38.3 us per step).  It still triggers its own successor (the next forward launch, one CTA per SM).
-        chamfer_grad_kernel<0><<<(unsigned int)blocks, 256, 0, stream>>>(p);
+        chamfer_grad_kernel<0, false><<<(unsigned int)blocks, 256, 0, stream>>>(p);
         return cudaGetLastError();
     }
     // two plain launches: stream order is the barrier between the stores and the atomics
-    chamfer_grad_kernel<2><<<(unsigned int)blocks, 256, 0, stream>>>(p);
-    chamfer_grad_kernel<3><<<(unsigned int)blocks, 256, 0, stream>>>(p);
+    chamfer_grad_kernel<2, false><<<(unsigned int)blocks, 256, 0, stream>>>(p);
+    chamfer_grad_kernel<3, false><<<(unsigned int)blocks, 256, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

@@ -1,6 +1,8 @@
 // chamfer_nn.cuh -- launch description shared by the two Chamfer NN forward kernels
 // (chamfer.cu: FFMA kernel for small launches; chamfer_nn_tc.cu: tensor-core kernel).
 #pragma once
+#include <type_traits>
+
 #include "psd_common.cuh"
 
 namespace psd {
@@ -48,6 +50,23 @@ struct NNParams {
     // and waiting for its predecessor would hold an SM that another stream's launch could use.
     int pdl_trigger;
 };
+
+// Ragged launches (the RAGGED instantiations of both NN kernels): pair c takes part with the first qlen[d][c] queries and
+// tlen[d][c] targets of direction d (device int [B]; NULL = the padded size).  The work grid stays that of the padded sizes.
+struct NNRaggedParams : NNParams {
+    const int *qlen[2], *tlen[2];
+};
+
+// participating queries / targets of pair `cloud` in direction d; a pair with a length outside [1, padded size] in either
+// cloud is invalid and gets qn = tn = 0
+__device__ __forceinline__ bool ragged_lengths(const NNRaggedParams &p, int d, int cloud, int &qn, int &tn) {
+    const NNDirection &D = p.dir[d];
+    qn = p.qlen[d] ? __ldg(p.qlen[d] + cloud) : D.nq;
+    tn = p.tlen[d] ? __ldg(p.tlen[d] + cloud) : D.nt;
+    const bool ok = qn >= 1 && qn <= D.nq && tn >= 1 && tn <= D.nt;
+    if (!ok) { qn = 0; tn = 0; }
+    return ok;
+}
 
 // grid-wide zero fill of p.zero_buf, a few stores per thread, issued before anything else in the forward kernels
 __device__ __forceinline__ void zero_fill(const NNParams &p) {

@@ -261,9 +261,21 @@ __device__ __forceinline__ float min32(const uint32_t (&r)[32]) {
 struct Unit {
     int d, cloud, qblock;
     int ttile, t0, nt;     // target tile of the unit: index, first target, number of targets (<= kMaxT)
+    int qn, tn, inval;     // ragged launches only: the pair's participating queries / targets (0 / 0 for an invalid pair)
 };
+template <class P> constexpr bool kRagged = std::is_same_v<P, NNRaggedParams>;
+// Ragged launches: the pair's lengths (reload) and the unit's target count.  A unit whose query block or target tile starts
+// at or beyond the lengths, or whose pair is invalid, gets nt = 0: the MMA thread, the scanners and the helpers all derive
+// their tile count from nt, so every role skips it by the same rule and the barrier phases stay in step.
+__device__ __forceinline__ void ragged_unit(const NNRaggedParams &p, Unit &u, bool reload) {
+    const NNDirection &D = p.dir[u.d];
+    if (reload) u.inval = !ragged_lengths(p, u.d, u.cloud, u.qn, u.tn);
+    u.nt = min(kMaxT, u.tn - u.t0);
+    if (u.nt < 0 || D.q_begin + u.qblock * kQB >= u.qn) u.nt = 0;
+}
 // unit order inside a direction: cloud, target tile, query block -- consecutive units of a CTA share a B operand
-__device__ __forceinline__ Unit decode_unit(const NNParams &p, int blk) {
+template <class P>
+__device__ __forceinline__ Unit decode_unit(const P &p, int blk) {
     Unit u;
     u.d = blk >= p.blocks_dir0 ? 1 : 0;
     const NNDirection &D = p.dir[u.d];
@@ -275,18 +287,31 @@ __device__ __forceinline__ Unit decode_unit(const NNParams &p, int blk) {
     u.qblock = rem - u.ttile * D.qblocks;
     u.t0 = u.ttile * kMaxT;
     u.nt = min(kMaxT, D.nt - u.t0);
+    if constexpr (kRagged<P>) ragged_unit(p, u, true);
     return u;
 }
 // unit blk -> unit blk + 1 without the integer divisions of decode_unit (they cost the single MMA thread ~500 cycles per unit)
-__device__ __forceinline__ void advance_unit(const NNParams &p, Unit &u, int blk_next) {
+template <class P>
+__device__ __forceinline__ void advance_unit(const P &p, Unit &u, int blk_next) {
     if (blk_next == p.blocks_dir0) { u = decode_unit(p, blk_next); return; }   // direction switch
     const NNDirection &D = p.dir[u.d];
     if (++u.qblock == D.qblocks) {
         u.qblock = 0;
+        const int cloud = u.cloud;
         if (++u.ttile == D.ntt) { u.ttile = 0; ++u.cloud; }
         u.t0 = u.ttile * kMaxT;
         u.nt = min(kMaxT, D.nt - u.t0);
+        if constexpr (kRagged<P>) ragged_unit(p, u, u.cloud != cloud);
+    } else if constexpr (kRagged<P>) {
+        ragged_unit(p, u, false);
     }
+}
+// last query of the unit's cloud that its query loads may touch (they are clamped to it); ragged: the last participating one
+template <class P>
+__device__ __forceinline__ int query_last(const P &p, const Unit &u) {
+    const NNDirection &D = p.dir[u.d];
+    if constexpr (kRagged<P>) return max(min(D.q_begin + D.q_count, u.qn) - 1, 0);
+    return D.q_begin + D.q_count - 1;
 }
 __device__ __forceinline__ int group_of(const NNParams &p, const Unit &u) { return u.d * 0x40000000 + u.cloud * p.dir[u.d].ntt + u.ttile; }
 __device__ __forceinline__ const float *targets_of(const NNParams &p, const Unit &u) {
@@ -317,7 +342,8 @@ struct FbQuery {
     const float *bx, *by, *bz;   // generic view of the targets: component base pointers and point stride
     long long ps;
 };
-__device__ __forceinline__ FbQuery fallback_query(const NNParams &p, int blk_begin, int e, const float *sraw, const int *s_rawgroup,
+template <class P>
+__device__ __forceinline__ FbQuery fallback_query(const P &p, int blk_begin, int e, const float *sraw, const int *s_rawgroup,
                                                   const float *fq) {   // fq: the query's coordinates in the list (x, y, z kFbCap apart)
     FbQuery q;
     q.u = decode_unit(p, blk_begin + ((e & 0x3fffffff) >> 8));
@@ -396,7 +422,8 @@ __device__ __forceinline__ void fallback_write(const NNParams &p, const FbQuery 
     if (p.fs_count && dres < p.fs_thr) atomicAdd(p.fs_count + q.u.cloud * 2 + D.slot, 1);
 }
 // one warp per query (used by the helpers when the list has to be flushed in the middle of the kernel)
-__device__ __forceinline__ void run_fallbacks(const NNParams &p, int blk_begin, const int *fb_list, const float *fb_q, int nfb, int wi, int nw,
+template <class P>
+__device__ __forceinline__ void run_fallbacks(const P &p, int blk_begin, const int *fb_list, const float *fb_q, int nfb, int wi, int nw,
                                               int lane, const float *sraw, const int *s_rawgroup) {
     for (int fi = wi; fi < nfb; fi += nw) {
         const FbQuery q = fallback_query(p, blk_begin, fb_list[fi], sraw, s_rawgroup, fb_q + fi);
@@ -407,8 +434,10 @@ __device__ __forceinline__ void run_fallbacks(const NNParams &p, int blk_begin, 
 
 // DBG: instrumented build -- dumps every filter value to dbg[(unit*128 + row) * dbg_ld + target] when dbg != nullptr
 // (calibration / bring-up) and writes phase clocks to prof (tools/tc_phase_clocks.py) when prof != nullptr.
-template <bool DBG>
-__global__ void __launch_bounds__(kThreadsTC, 1) chamfer_nn_tc_kernel(const NNParams p, float *dbg, int dbg_ld, long long *prof) {
+// RAGGED: per-pair lengths (NNRaggedParams); the units of the padded grid that lie beyond them do no search.
+template <bool DBG, bool RAGGED>
+__global__ void __launch_bounds__(kThreadsTC, 1) chamfer_nn_tc_kernel(const std::conditional_t<RAGGED, NNRaggedParams, NNParams> p,
+                                                                     float *dbg, int dbg_ld, long long *prof) {
     extern __shared__ __align__(128) unsigned char smem[];
     float *sraw = reinterpret_cast<float *>(smem + kOffRaw);
     float *part = reinterpret_cast<float *>(smem + kOffPart);
@@ -576,7 +605,7 @@ __global__ void __launch_bounds__(kThreadsTC, 1) chamfer_nn_tc_kernel(const NNPa
         if (tid >= kHelp0 && tid - kHelp0 < kQB) {
             // the queries of unit 0 travel together with its targets: one global round trip on the critical path, not two
             int j = D.q_begin + u.qblock * kQB + (tid - kHelp0);
-            const int q_last = D.q_begin + D.q_count - 1;
+            const int q_last = query_last(p, u);
             j = j < q_last ? j : q_last;
             const float *qp = D.q + (long long)u.cloud * D.q_bs + j * D.q_ps;
             pq1 = __ldg(qp); pq2 = __ldg(qp + D.q_cs); pq3 = __ldg(qp + 2 * D.q_cs);
@@ -608,6 +637,10 @@ __global__ void __launch_bounds__(kThreadsTC, 1) chamfer_nn_tc_kernel(const NNPa
         for (int ul = 0; ul < nunits; ++ul) {
             if (ul > 0) advance_unit(p, u, blk_begin + ul);
             const int ntiles = (u.nt + kTileN - 1) / kTileN;
+            // A unit without tiles (ragged launches) has no MMA to pace the scanners: without this wait they could park its
+            // partials in the slot of unit ul - 2 and arrive on that slot's barrier before the helpers have resolved unit
+            // ul - 2.  Its operands are staged (bar_ready) only after that resolve.
+            if (RAGGED && ntiles == 0) mbar_wait_warp(bar_ready + 8 * (ul & 1), (ul >> 1) & 1, s_abort);
             float best = kBig, second = kBig;
             int bchunk = 0;
             auto chunk = [&](const uint32_t (&v)[32], int cid) {
@@ -794,7 +827,7 @@ __global__ void __launch_bounds__(kThreadsTC, 1) chamfer_nn_tc_kernel(const NNPa
             const NNDirection &D = p.dir[u.d];
             if (ht < kQB && ul > 0) {   // (unit 0's queries were loaded in the prologue)
                 int j = D.q_begin + u.qblock * kQB + ht;
-                const int q_last = D.q_begin + D.q_count - 1;
+                const int q_last = query_last(p, u);
                 j = j < q_last ? j : q_last;
                 const float *qp = D.q + (long long)u.cloud * D.q_bs + j * D.q_ps;
                 pq1 = __ldg(qp); pq2 = __ldg(qp + D.q_cs); pq3 = __ldg(qp + 2 * D.q_cs);
@@ -856,7 +889,8 @@ __global__ void __launch_bounds__(kThreadsTC, 1) chamfer_nn_tc_kernel(const NNPa
             // ---- A
             const int ql = q0 + (lane < nqw ? lane : 0);
             const int j = D.q_begin + u.qblock * kQB + ql;
-            const bool live = lane < nqw && j < D.q_begin + D.q_count;
+            // (ragged: a unit without targets -- a tile beyond the pair's targets in multi-tile mode -- has nothing to search)
+            const bool live = lane < nqw && j < D.q_begin + D.q_count && (!RAGGED || (j < u.qn && u.nt > 0));
             float b1 = kBig, b2 = kBig;
             int bc = 0;
 #pragma unroll
@@ -891,6 +925,16 @@ __global__ void __launch_bounds__(kThreadsTC, 1) chamfer_nn_tc_kernel(const NNPa
             const bool ok = live && !fr.bad && (qn < kQMax) && (b2 > b1 + margin);
             float ws = 0.f;   // fused epilogue accumulators of this lane
             int wc = 0;
+            if constexpr (RAGGED) {
+                // rows past the pair's query length, and every row of an invalid pair: dist 0 (NaN), idx -1, counted nowhere
+                // (the NaN goes into the pair's sums); the multi-tile mode leaves them to the finalize kernel
+                if (lane < nqw && j < D.q_begin + D.q_count && !live && D.ws == nullptr) {
+                    const float dz = u.inval ? __int_as_float(0x7fc00000) : 0.f;
+                    D.dist[(long long)u.cloud * D.nq + j] = dz;
+                    D.idx[(long long)u.cloud * D.nq + j] = -1;
+                    ws += dz;
+                }
+            }
             if (DBG && ht == 0) stamp(12 + ul * 6);
             // ---- B
 #pragma unroll
@@ -1072,7 +1116,10 @@ using namespace psd;
 // (a NaN distance to target 0 poisons the result: chamfer3D.cu:36,126) and the fused loss-sum / F-score epilogue.
 namespace psd {
 namespace tc {
-__global__ void __launch_bounds__(256) chamfer_nn_tc_finalize_kernel(const NNParams p, int b) {
+// RAGGED: rows past the pair's query length get dist 0, idx -1 and are not counted; every row of an invalid pair gets NaN, -1.
+template <bool RAGGED>
+__global__ void __launch_bounds__(256) chamfer_nn_tc_finalize_kernel(const std::conditional_t<RAGGED, NNRaggedParams, NNParams> p,
+                                                                     int b) {
     const long long n0 = p.dir[0].ws ? (long long)b * p.dir[0].q_count : 0;
     const long long n1 = p.dir[1].ws ? (long long)b * p.dir[1].q_count : 0;
     const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1081,17 +1128,27 @@ __global__ void __launch_bounds__(256) chamfer_nn_tc_finalize_kernel(const NNPar
     const NNDirection &D = p.dir[d];
     float dres = 0.f;
     int cloud = -1;
+    bool counted = active;
     if (active) {
         const long long e = d ? gid - n0 : gid;
         cloud = (int)(e / D.q_count);
         const int j = D.q_begin + (int)(e - (long long)cloud * D.q_count);
         const unsigned long long key = D.ws[(long long)cloud * D.nq + j];
         D.ws[(long long)cloud * D.nq + j] = ~0ull;   // the library-owned workspace is always left clean for the next launch
-        const float *qp = D.q + (long long)cloud * D.q_bs + (long long)j * D.q_ps;
-        const float d0 = exact_d(D.t + (long long)cloud * D.t_bs, D.t_ps, D.t_cs, 0, __ldg(qp), __ldg(qp + D.q_cs), __ldg(qp + 2 * D.q_cs));
+        int qn = 0, tn = 0;
+        bool ok = true;
+        if constexpr (RAGGED) ok = ragged_lengths(p, d, cloud, qn, tn);
         int ires;
-        if (d0 != d0) { dres = d0; ires = 0; }
-        else { dres = __uint_as_float((unsigned int)(key >> 32)); ires = (int)(key & 0xffffffffu); }
+        if (RAGGED && j >= qn) {   // (the query row itself is never read)
+            dres = ok ? 0.f : __int_as_float(0x7fc00000);
+            ires = -1;
+            counted = false;
+        } else {
+            const float *qp = D.q + (long long)cloud * D.q_bs + (long long)j * D.q_ps;
+            const float d0 = exact_d(D.t + (long long)cloud * D.t_bs, D.t_ps, D.t_cs, 0, __ldg(qp), __ldg(qp + D.q_cs), __ldg(qp + 2 * D.q_cs));
+            if (d0 != d0) { dres = d0; ires = 0; }
+            else { dres = __uint_as_float((unsigned int)(key >> 32)); ires = (int)(key & 0xffffffffu); }
+        }
         D.dist[(long long)cloud * D.nq + j] = dres;
         D.idx[(long long)cloud * D.nq + j] = ires;
     }
@@ -1101,7 +1158,7 @@ __global__ void __launch_bounds__(256) chamfer_nn_tc_finalize_kernel(const NNPar
         const int k0 = __shfl_sync(0xffffffffu, key2, 0);
         const bool uniform = __all_sync(0xffffffffu, key2 == k0);
         float ws = active ? dres : 0.f;
-        int wc = (active && dres < p.fs_thr) ? 1 : 0;
+        int wc = (counted && dres < p.fs_thr) ? 1 : 0;
         if (uniform) {
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) { ws += __shfl_xor_sync(0xffffffffu, ws, o); wc += __shfl_xor_sync(0xffffffffu, wc, o); }
@@ -1184,12 +1241,15 @@ static cudaError_t acquire_merge_ws(DeviceState *ds, cudaStream_t stream, size_t
     return cudaSuccess;
 }
 
-cudaError_t psd_launch_nn_tc(const NNParams &p_in, DeviceState *ds, cudaStream_t stream, float *dbg, int dbg_ld, long long *prof, int b) {
+// ragged: per-pair lengths len1 / len2 of xyz1 / xyz2 (device int [b], NULL = n / m), see NNRaggedParams
+cudaError_t psd_launch_nn_tc(const NNParams &p_in, DeviceState *ds, cudaStream_t stream, float *dbg, int dbg_ld, long long *prof, int b,
+                             bool ragged, const int *len1, const int *len2) {
     {
         std::lock_guard<std::mutex> lock(state_mutex());
         if (!ds->attr_tc) {
-            cudaError_t e = cudaFuncSetAttribute(tc::chamfer_nn_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemTC);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::chamfer_nn_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemTC);
+            cudaError_t e = cudaFuncSetAttribute(tc::chamfer_nn_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemTC);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::chamfer_nn_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemTC);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::chamfer_nn_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemTC);
             if (e != cudaSuccess) return e;
             ds->attr_tc = true;
         }
@@ -1225,14 +1285,20 @@ cudaError_t psd_launch_nn_tc(const NNParams &p_in, DeviceState *ds, cudaStream_t
     const int cap = g_tc_max_ctas.load();
     if (cap > 0 && grid > cap) grid = cap;
     p.pdl_trigger = (cap > 0 && grid == cap) ? 0 : 1;
+    NNRaggedParams pr;
+    static_cast<NNParams &>(pr) = p;
+    pr.qlen[0] = len1; pr.tlen[0] = len2;   // direction 0: xyz1 -> xyz2
+    pr.qlen[1] = len2; pr.tlen[1] = len1;
     cudaError_t e;
-    if (dbg || prof) e = psd_launch_pdl(p.pdl_trigger != 0, tc::chamfer_nn_tc_kernel<true>, dim3(grid), dim3(tc::kThreadsTC), tc::kSmemTC, stream, p, dbg, dbg_ld, prof);
-    else e = psd_launch_pdl(p.pdl_trigger != 0, tc::chamfer_nn_tc_kernel<false>, dim3(grid), dim3(tc::kThreadsTC), tc::kSmemTC, stream, p, (float *)nullptr, 0, (long long *)nullptr);
+    if (ragged) e = psd_launch_pdl(p.pdl_trigger != 0, tc::chamfer_nn_tc_kernel<false, true>, dim3(grid), dim3(tc::kThreadsTC), tc::kSmemTC, stream, pr, (float *)nullptr, 0, (long long *)nullptr);
+    else if (dbg || prof) e = psd_launch_pdl(p.pdl_trigger != 0, tc::chamfer_nn_tc_kernel<true, false>, dim3(grid), dim3(tc::kThreadsTC), tc::kSmemTC, stream, p, dbg, dbg_ld, prof);
+    else e = psd_launch_pdl(p.pdl_trigger != 0, tc::chamfer_nn_tc_kernel<false, false>, dim3(grid), dim3(tc::kThreadsTC), tc::kSmemTC, stream, p, (float *)nullptr, 0, (long long *)nullptr);
     if (ws_elems) {
         if (e == cudaSuccess) {
             const long long total = (p.dir[0].ws ? (long long)b * p.dir[0].q_count : 0) + (p.dir[1].ws ? (long long)b * p.dir[1].q_count : 0);
             if (total > 0) {
-                tc::chamfer_nn_tc_finalize_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(p, b);
+                if (ragged) tc::chamfer_nn_tc_finalize_kernel<true><<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(pr, b);
+                else tc::chamfer_nn_tc_finalize_kernel<false><<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(p, b);
                 e = cudaGetLastError();
             }
         }

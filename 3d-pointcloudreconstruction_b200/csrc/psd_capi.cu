@@ -12,11 +12,13 @@
 cudaError_t psd_launch_chamfer_forward(const float *xyz1, const float *xyz2, int b, int n, int m, int layout,
                                        float *dist1, float *dist2, int *idx1, int *idx2, float *sums, float fs_thr,
                                        int *fs_count, int q_begin, int q_count, cudaStream_t stream, float *zero_buf = nullptr,
-                                       long long zero_floats = 0);
+                                       long long zero_floats = 0, bool ragged = false, const int *len1 = nullptr,
+                                       const int *len2 = nullptr);
 cudaError_t psd_launch_chamfer_backward(const float *xyz1, const float *xyz2, float *gradxyz1, float *gradxyz2,
                                         const float *graddist1, const float *graddist2, const int *idx1, const int *idx2,
                                         int b, int n, int m, int layout, int overwrite, cudaStream_t stream,
-                                        const float *upstream = nullptr);
+                                        const float *upstream = nullptr, bool ragged = false, const int *len1 = nullptr,
+                                        const int *len2 = nullptr);
 cudaError_t psd_launch_chamfer_mean_loss(const float *sums, int b, int n, int m, float *out, cudaStream_t stream);
 cudaError_t psd_read_chamfer_stats(unsigned long long *fallback, int reset);
 int psd_set_nn_variant(int v);
@@ -148,6 +150,30 @@ int psd_chamfer_backward_ex(const float *xyz1, const float *xyz2, float *gradxyz
     return finish("psd_chamfer_backward_ex",
                   psd_launch_chamfer_backward(xyz1, xyz2, gradxyz1, gradxyz2, graddist1, graddist2, idx1, idx2, b, n, m,
                                               layout, overwrite != 0, (cudaStream_t)stream));
+}
+
+int psd_chamfer_forward_ragged(const float *xyz1, const float *xyz2, int b, int n, int m, int layout, const int *len1,
+                               const int *len2, float *dist1, float *dist2, int *idx1, int *idx2, float *sums, float fs_thr,
+                               int *fs_count, float *zero_buf, long long zero_floats, void *stream) {
+    if (layout < 0 || layout > 3) {
+        psd_set_error_msg("psd_chamfer_forward_ragged: layout is a bit mask: 1 = xyz1 is [B,3,N], 2 = xyz2 is [B,3,M]");
+        return -1;
+    }
+    return finish("psd_chamfer_forward_ragged",
+                  psd_launch_chamfer_forward(xyz1, xyz2, b, n, m, layout, dist1, dist2, idx1, idx2, sums, fs_thr, fs_count, 0,
+                                             -1, (cudaStream_t)stream, zero_buf, zero_floats, true, len1, len2));
+}
+
+int psd_chamfer_backward_ragged(const float *xyz1, const float *xyz2, float *gradxyz1, float *gradxyz2,
+                                const float *graddist1, const float *graddist2, const int *idx1, const int *idx2,
+                                const int *len1, const int *len2, int b, int n, int m, int layout, void *stream) {
+    if (layout < 0 || layout > 3) {
+        psd_set_error_msg("psd_chamfer_backward_ragged: layout is a bit mask: 1 = xyz1 is [B,3,N], 2 = xyz2 is [B,3,M]");
+        return -1;
+    }
+    return finish("psd_chamfer_backward_ragged",
+                  psd_launch_chamfer_backward(xyz1, xyz2, gradxyz1, gradxyz2, graddist1, graddist2, idx1, idx2, b, n, m,
+                                              layout, 0, (cudaStream_t)stream, nullptr, true, len1, len2));
 }
 
 static const char *kEmdShapeMsg = "the cloud size must be a multiple of the cluster size";

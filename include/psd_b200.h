@@ -83,6 +83,25 @@ int psd_chamfer_backward_ex(const float *xyz1, const float *xyz2, float *gradxyz
                             const float *graddist1, const float *graddist2, const int *idx1, const int *idx2, int b, int n,
                             int m, int layout, int overwrite, void *stream);
 
+/* Ragged batches in one launch.  xyz1 [b, n, 3] and xyz2 [b, m, 3] are padded (layout as psd_chamfer_forward_ex); pair c
+ * takes part with its first len1[c] points of xyz1 and len2[c] points of xyz2 (device int [b]; NULL = n / m for every pair).
+ * Points beyond the lengths are never read (they may hold NaN, inf or garbage).  dist / idx of pair c are the bits of
+ * psd_chamfer_forward on its participating points alone (lowest index on ties, the reference's 512-target NaN rule);
+ * rows beyond the lengths get dist 0 and idx -1 and add nothing to sums / fs_count (optional [b, 2], caller-zeroed, as in
+ * psd_chamfer_forward_ex).  A pair with a length outside [1, n] / [1, m] gets dist NaN and idx -1 in every row, NaN sums
+ * and zero counts, without affecting the others.  zero_buf / zero_floats: as in psd_chamfer_forward_zero.  The launch
+ * grid is that of the padded sizes and the lengths are read on the device only: no host synchronisation, graph-capturable.
+ * psd_chamfer_nn_variant applies.  Returns -1 for a bad layout, else the convention above. */
+int psd_chamfer_forward_ragged(const float *xyz1, const float *xyz2, int b, int n, int m, int layout, const int *len1,
+                               const int *len2, float *dist1, float *dist2, int *idx1, int *idx2, float *sums, float fs_thr,
+                               int *fs_count, float *zero_buf, long long zero_floats, void *stream);
+/* The gradient of psd_chamfer_forward_ragged, accumulated into caller-zeroed buffers (psd_chamfer_backward's form, e.g. the
+ * buffers the ragged forward zero-filled).  Rows beyond the lengths get no term (their gradient stays 0) and their graddist
+ * entries are never read; every gradient row of a pair with an invalid length becomes NaN. */
+int psd_chamfer_backward_ragged(const float *xyz1, const float *xyz2, float *gradxyz1, float *gradxyz2,
+                                const float *graddist1, const float *graddist2, const int *idx1, const int *idx2,
+                                const int *len1, const int *len2, int b, int n, int m, int layout, void *stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Earth mover's distance, auction approximation.
  * ------------------------------------------------------------------------------------------- */
