@@ -64,6 +64,7 @@ _SIGNATURES = {
     "psd_chamfer_tc_ctas": [_ci],
     "psd_proj_min_dist": [_vp, _vp, _vp, _ci, _ci, _ci, _ci, _vp, _vp, _vp],
     "psd_icp_batch": [_vp, _vp, _ci, _ci, _ci, _vp, _ci, ctypes.c_double, _vp, _vp, _vp, _vp],
+    "psd_icp_batch_ragged": [_vp, _vp, _ci, _ci, _ci, _ci, _vp, _vp, _vp, _ci, ctypes.c_double, _vp, _vp, _vp, _vp],
     "psd_nn_f64": [_vp, _vp, _ci, _ci, _ci, _ci, _vp, _vp, _vp],
     "psd_farthest_point_sample": [_vp, _ci, _ci, _ci, _ci, _vp, _vp],
     "psd_cont_proj": [_vp, _ci, _ci, _ci, _ci, ctypes.c_float, _vp, _vp],

@@ -11,6 +11,10 @@
 //                                         det R < 0) is the proper-rotation completion u3 = u1 x u2, v3 = v1 x v2
 //     src = T src, mean error, |prev - mean| < tolerance -> break (:103-110), final T = best_fit_transform(A, src) (:113)
 // All arithmetic is fp64 like numpy's; inputs are fp32 (what the callers pass; the conversion is exact) or fp64.
+// Ragged batches (psd_icp_batch_ragged): sample s aligns its first len_a[s] source points to its first len_b[s] destination
+// points (any two sizes, as the reference's icp() allows without its shape assert); the uniform instantiations are unchanged.
+#include <type_traits>
+
 #include "psd_common.cuh"
 
 namespace psd {
@@ -27,6 +31,12 @@ struct IcpParams {
     double *T;                // [batch, 4, 4]
     double *dist;             // [batch, n] distances of the last NN pass (may be null)
     int *iters;               // [batch] the reference's `i` (may be null)
+};
+
+// a, dist: [batch, n, *] and b: [batch, m, 3] padded; a sample takes part with its first len_a / len_b points
+struct IcpRaggedParams : IcpParams {
+    int m;                    // padded destination size
+    const int *len_a, *len_b; // [batch] device (NULL = n / m)
 };
 
 __device__ __forceinline__ double ld_coord(const void *p, int f64, long long i) {
@@ -138,30 +148,55 @@ __device__ void transform_from_sums(const double *cA, const double *cB, const do
     T[12] = 0.0; T[13] = 0.0; T[14] = 0.0; T[15] = 1.0;
 }
 
-// Q = source points per thread (n <= Q * 512)
-template <int Q>
-__global__ void __launch_bounds__(kIcpThreads, 1) icp_kernel(IcpParams p) {
+// the sample's source / destination point counts and the padded destination size
+__device__ __forceinline__ int src_count(const IcpParams &p, int) { return p.n; }
+__device__ __forceinline__ int dst_count(const IcpParams &p, int) { return p.n; }
+__device__ __forceinline__ int dst_stride(const IcpParams &p) { return p.n; }
+__device__ __forceinline__ int src_count(const IcpRaggedParams &p, int s) { return p.len_a ? p.len_a[s] : p.n; }
+__device__ __forceinline__ int dst_count(const IcpRaggedParams &p, int s) { return p.len_b ? p.len_b[s] : p.m; }
+__device__ __forceinline__ int dst_stride(const IcpRaggedParams &p) { return p.m; }
+
+// Q = source points per thread (n <= Q * 512).  RAGGED (IcpRaggedParams): n below is the sample's own source count and nb its
+// destination count; Q still comes from the padded n, so thread tid owns the points tid + r*512 in the same order as in a
+// uniform launch on the sample alone, and the slots beyond the count are skipped as there: the results are its bits.
+template <int Q, bool RAGGED>
+__global__ void __launch_bounds__(kIcpThreads, 1) icp_kernel(const std::conditional_t<RAGGED, IcpRaggedParams, IcpParams> p) {
     extern __shared__ double smd[];
-    const int n = p.n, tid = threadIdx.x, sample = blockIdx.x;
-    double *sx = smd, *sy = sx + n, *sz = sy + n, *tx = sz + n, *ty = tx + n, *tz = ty + n;
-    double *red = tz + n;            // 16 warps * 9 (sized for 32)
+    const int sample = blockIdx.x;
+    const int n = src_count(p, sample), nb = dst_count(p, sample), tid = threadIdx.x;
+    if constexpr (RAGGED) {
+        if (!(n >= 1 && n <= p.n && nb >= 1 && nb <= p.m)) {   // invalid lengths: NaN, -1, none of the points read
+            const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+            if (tid < 16) p.T[(long long)sample * 16 + tid] = qnan;
+            if (p.dist)
+                for (int j = tid; j < p.n; j += kIcpThreads) p.dist[(long long)sample * p.n + j] = qnan;
+            if (p.iters && tid == 0) p.iters[sample] = -1;
+            return;
+        }
+    }
+    double *sx = smd, *sy = sx + n, *sz = sy + n, *tx = sz + n, *ty = tx + nb, *tz = ty + nb;
+    double *red = tz + nb;           // 16 warps * 9 (sized for 32)
     double *tot = red + 32 * 9;      // 9 totals
     double *sT = tot + 9;            // 12 + flag
-    const long long base = (long long)sample * n * 3;
+    const long long base = (long long)sample * p.n * 3, bbase = (long long)sample * dst_stride(p) * 3;
 
-    for (int j = tid; j < n; j += kIcpThreads) {
-        double x = ld_coord(p.a, p.in_f64, base + 3 * j), y = ld_coord(p.a, p.in_f64, base + 3 * j + 1),
-               z = ld_coord(p.a, p.in_f64, base + 3 * j + 2);
-        if (p.init_pose && p.max_iter > 0) {
-            const double *P = p.init_pose;
-            const double nx = P[0] * x + P[1] * y + P[2] * z + P[3], ny = P[4] * x + P[5] * y + P[6] * z + P[7],
-                         nz = P[8] * x + P[9] * y + P[10] * z + P[11];
-            x = nx; y = ny; z = nz;
+    for (int j = tid; j < (RAGGED ? max(n, nb) : n); j += kIcpThreads) {
+        if (!RAGGED || j < n) {
+            double x = ld_coord(p.a, p.in_f64, base + 3 * j), y = ld_coord(p.a, p.in_f64, base + 3 * j + 1),
+                   z = ld_coord(p.a, p.in_f64, base + 3 * j + 2);
+            if (p.init_pose && p.max_iter > 0) {
+                const double *P = p.init_pose;
+                const double nx = P[0] * x + P[1] * y + P[2] * z + P[3], ny = P[4] * x + P[5] * y + P[6] * z + P[7],
+                             nz = P[8] * x + P[9] * y + P[10] * z + P[11];
+                x = nx; y = ny; z = nz;
+            }
+            sx[j] = x; sy[j] = y; sz[j] = z;
         }
-        sx[j] = x; sy[j] = y; sz[j] = z;
-        tx[j] = ld_coord(p.b, p.in_f64, base + 3 * j);
-        ty[j] = ld_coord(p.b, p.in_f64, base + 3 * j + 1);
-        tz[j] = ld_coord(p.b, p.in_f64, base + 3 * j + 2);
+        if (!RAGGED || j < nb) {
+            tx[j] = ld_coord(p.b, p.in_f64, bbase + 3 * j);
+            ty[j] = ld_coord(p.b, p.in_f64, bbase + 3 * j + 1);
+            tz[j] = ld_coord(p.b, p.in_f64, bbase + 3 * j + 2);
+        }
     }
     __syncthreads();
 
@@ -187,7 +222,7 @@ __global__ void __launch_bounds__(kIcpThreads, 1) icp_kernel(IcpParams p) {
                 bidx[r] = 0;
             }
 #pragma unroll 2
-            for (int k = 0; k < n; ++k) {
+            for (int k = 0; k < nb; ++k) {
                 const double kx = tx[k], ky = ty[k], kz = tz[k];
 #pragma unroll
                 for (int r = 0; r < Q; ++r) {
@@ -250,7 +285,11 @@ __global__ void __launch_bounds__(kIcpThreads, 1) icp_kernel(IcpParams p) {
 #pragma unroll
         for (int r = 0; r < Q; ++r) {
             const int j = tid + r * kIcpThreads;
-            if (j < n) p.dist[(long long)sample * n + j] = best[r];
+            if constexpr (RAGGED) {
+                if (j < p.n) p.dist[(long long)sample * p.n + j] = j < n ? best[r] : 0.0;
+            } else {
+                if (j < n) p.dist[(long long)sample * n + j] = best[r];
+            }
         }
     }
     if (p.iters && tid == 0) p.iters[sample] = it_out;
@@ -341,7 +380,27 @@ cudaError_t psd_launch_icp(const void *a, const void *b, int in_f64, int batch, 
     IcpParams p{a, b, in_f64, init_pose, batch, n, max_iter, tol, T, dist, iters};
     const size_t smem = sizeof(double) * ((size_t)6 * n + 32 * 9 + 9 + 16);
     const int q = (n + kIcpThreads - 1) / kIcpThreads;
-    void (*kern)(IcpParams) = q <= 1 ? icp_kernel<1> : q <= 2 ? icp_kernel<2> : q <= 4 ? icp_kernel<4> : icp_kernel<8>;
+    void (*kern)(IcpParams) = q <= 1 ? icp_kernel<1, false> : q <= 2 ? icp_kernel<2, false>
+                            : q <= 4 ? icp_kernel<4, false> : icp_kernel<8, false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kern<<<batch, kIcpThreads, smem, stream>>>(p);
+    return cudaGetLastError();
+}
+
+// n <= 4096 (Q <= 8), n + m <= 8192 (the fp64 SoA clouds take the shared memory of the uniform n = 4096), max_iter >= 1
+cudaError_t psd_launch_icp_ragged(const void *a, const void *b, int in_f64, int batch, int n, int m, const int *len_a,
+                                  const int *len_b, const double *init_pose, int max_iter, double tol, double *T, double *dist,
+                                  int *iters, cudaStream_t stream) {
+    using namespace psd;
+    if (batch <= 0) return cudaSuccess;
+    IcpRaggedParams p;
+    static_cast<IcpParams &>(p) = IcpParams{a, b, in_f64, init_pose, batch, n, max_iter, tol, T, dist, iters};
+    p.m = m; p.len_a = len_a; p.len_b = len_b;
+    const size_t smem = sizeof(double) * ((size_t)3 * (n + m) + 32 * 9 + 9 + 16);
+    const int q = (n + kIcpThreads - 1) / kIcpThreads;
+    void (*kern)(IcpRaggedParams) = q <= 1 ? icp_kernel<1, true> : q <= 2 ? icp_kernel<2, true>
+                                  : q <= 4 ? icp_kernel<4, true> : icp_kernel<8, true>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kern<<<batch, kIcpThreads, smem, stream>>>(p);

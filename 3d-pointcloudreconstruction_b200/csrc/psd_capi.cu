@@ -26,6 +26,9 @@ cudaError_t psd_launch_icp(const void *a, const void *b, int in_f64, int batch, 
                            double tol, double *T, double *dist, int *iters, cudaStream_t stream);
 cudaError_t psd_launch_nn_f64(const void *src, const void *dst, int in_f64, int batch, int n_src, int n_dst, double *distances,
                               int *indices, cudaStream_t stream);
+cudaError_t psd_launch_icp_ragged(const void *a, const void *b, int in_f64, int batch, int n, int m, const int *len_a,
+                                  const int *len_b, const double *init_pose, int max_iter, double tol, double *T, double *dist,
+                                  int *iters, cudaStream_t stream);
 int psd_icp_max_points();
 int psd_set_emd_solo(int enable);
 int psd_set_emd_grid(int enable);
@@ -413,6 +416,21 @@ int psd_icp_batch(const void *a, const void *b, int in_f64, int batch, int n, co
     if (n > psd_icp_max_points()) { psd_set_error_msg("psd_icp_batch: n exceeds the shared-memory resident limit (4096 points)"); return -1; }
     return finish("psd_icp_batch", psd_launch_icp(a, b, in_f64, batch, n, init_pose, max_iterations, tolerance, T_out, distances,
                                                   iterations, (cudaStream_t)stream));
+}
+
+int psd_icp_batch_ragged(const void *a, const void *b, int in_f64, int batch, int n, int m, const int *len_a, const int *len_b,
+                         const double *init_pose, int max_iterations, double tolerance, double *T_out, double *distances,
+                         int *iterations, void *stream) {
+    if (batch < 0 || n < 1 || m < 1 || max_iterations < 1) {
+        psd_set_error_msg("psd_icp_batch_ragged: batch >= 0, n >= 1, m >= 1, max_iterations >= 1 required");
+        return -1;
+    }
+    if (n > psd_icp_max_points() || n + m > 2 * psd_icp_max_points()) {
+        psd_set_error_msg("psd_icp_batch_ragged: n <= 4096 and n + m <= 8192 required (shared-memory resident clouds)");
+        return -1;
+    }
+    return finish("psd_icp_batch_ragged", psd_launch_icp_ragged(a, b, in_f64, batch, n, m, len_a, len_b, init_pose, max_iterations,
+                                                                tolerance, T_out, distances, iterations, (cudaStream_t)stream));
 }
 
 int psd_farthest_point_sample(const float *xyz, int b, int n, int npoint, int start, long long *centroids, void *stream) {

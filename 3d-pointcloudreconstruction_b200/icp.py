@@ -1,7 +1,7 @@
 """Drop-in for utils/icp.py: ``best_fit_transform(A, B)``, ``nearest_neighbor(src, dst)`` and
 ``icp(A, B, init_pose=None, max_iterations=20, tolerance=0.001)`` with the reference's signatures, numpy in / numpy out, plus
 ``icp_batch`` which aligns a whole batch of samples in one kernel launch (the reference's callers loop over the samples,
-testnet.py:62-64).
+testnet.py:62-64), and ``icp_ragged`` for a batch whose samples have their own source and destination sizes.
 
 The reference runs a sklearn KD-tree build + query, numpy reductions and a 3x3 SVD per iteration on the CPU; here the whole
 iteration loop of every sample runs inside one CUDA kernel (csrc/icp.cu, psd_icp_batch), in fp64 like numpy.  There is no
@@ -13,8 +13,13 @@ import torch
 
 try:
     from . import _lib
+    from .sinkhorn import _lengths
 except ImportError:
     import _lib
+    from sinkhorn import _lengths
+
+MAX_POINTS = 4096         # source points of one sample (padded N)
+MAX_POINTS_PAIR = 8192    # source + destination points of one sample (padded N + M)
 
 
 def _device():
@@ -50,6 +55,62 @@ def icp_batch(A, B, init_pose=None, max_iterations=20, tolerance=0.001):
                                     None if pose is None else _lib.ptr(pose), int(max_iterations), ctypes.c_double(tolerance),
                                     _lib.ptr(T), _lib.ptr(dist), _lib.ptr(iters), _lib.stream_of(a))
     _lib.raise_on_cuda_error(rc, "psd_icp_batch")
+    return T, dist, iters
+
+
+def icp_ragged(A, B, a_lengths=None, b_lengths=None, init_pose=None, max_iterations=20, tolerance=0.001):
+    """icp() for every sample of a ragged batch, in one launch: sample s aligns its first a_lengths[s] source points A[s] to
+    its first b_lengths[s] destination points B[s].  The two sizes need not be equal: the reference's algorithm is defined
+    for any sizes, only its ``assert A.shape == B.shape`` forbids them.
+
+    A [batch, N, 3] and B [batch, M, 3] are padded (numpy or torch, float32 or float64; mixed dtypes are promoted to
+    float64), with N <= 4096 and N + M <= 8192; a_lengths / b_lengths [batch] default to N / M.  Rows past the lengths are
+    never read.  A list or CPU tensor of lengths is checked here (ValueError unless every length is in [1, N] / [1, M]); a
+    CUDA integer tensor is used as it is, and a sample with a length out of range gets T all NaN, NaN distances and
+    iteration -1 without affecting the others.  max_iterations must be >= 1.
+
+    Returns (T [batch,4,4] float64, distances [batch,N] float64, iterations [batch] int32) on the device: T maps the source
+    onto the destination, distances are those of the last NN pass (0 past a_lengths[s]).  A sample with equal lengths gets
+    the bits ``icp_batch`` gives on its points alone.
+
+    The evaluation of scans of different sizes against fixed-size predictions, with the ground truth as the moving source
+    as in testnet.py:57-64, then runs in two launches::
+
+        gt, lengths = pack_clouds(scans)                          # [B, max k, 3], [B]
+        T, _, _ = icp_ragged(gt, preds, lengths, tolerance=1e-10, max_iterations=1024)
+        aligned = gt.double() @ T[:, :3, :3].transpose(1, 2) + T[:, None, :3, 3]
+        r = chamfer_fscore_fused(aligned.float(), preds, x_lengths=lengths)
+    """
+    a, b = torch.as_tensor(A), torch.as_tensor(B)
+    if a.dim() != 3 or a.shape[2] != 3 or b.dim() != 3 or b.shape[2] != 3 or a.shape[0] != b.shape[0]:
+        raise ValueError(f"A and B must be [batch, N, 3] and [batch, M, 3], got {tuple(a.shape)} and {tuple(b.shape)}")
+    batch, n, m = a.shape[0], a.shape[1], b.shape[1]
+    if n < 1 or m < 1 or n > MAX_POINTS or n + m > MAX_POINTS_PAIR:
+        raise ValueError(f"icp_ragged needs 1 <= N <= {MAX_POINTS} and N + M <= {MAX_POINTS_PAIR}, got N = {n}, M = {m}")
+    if max_iterations < 1:
+        raise ValueError("icp_ragged needs max_iterations >= 1")
+    la = None if a_lengths is None else _lengths("a_lengths", a_lengths, batch, n)
+    lb = None if b_lengths is None else _lengths("b_lengths", b_lengths, batch, m)
+    dev = a.device if a.is_cuda else _device()
+    a, b = _to_dev(a, dev), _to_dev(b, dev)
+    if a.dtype != b.dtype:
+        a, b = a.double(), b.double()
+    la = None if la is None else la.to(dev)
+    lb = None if lb is None else lb.to(dev)
+    pose = None if init_pose is None else torch.as_tensor(np.asarray(init_pose, dtype=np.float64)).to(dev).contiguous()
+    if pose is not None and pose.shape != (4, 4):
+        raise ValueError("init_pose must be 4x4")
+    T = torch.empty(batch, 4, 4, device=dev, dtype=torch.float64)
+    dist = torch.empty(batch, n, device=dev, dtype=torch.float64)
+    iters = torch.empty(batch, device=dev, dtype=torch.int32)
+    with torch.cuda.device(dev):
+        rc = _lib.lib.psd_icp_batch_ragged(_lib.ptr(a), _lib.ptr(b), int(a.dtype == torch.float64), batch, n, m, _lib.ptr(la),
+                                           _lib.ptr(lb), None if pose is None else _lib.ptr(pose), int(max_iterations),
+                                           ctypes.c_double(tolerance), _lib.ptr(T), _lib.ptr(dist), _lib.ptr(iters),
+                                           _lib.stream_of(a))
+    if rc == -1:
+        raise ValueError(_lib.last_error())
+    _lib.raise_on_cuda_error(rc, "psd_icp_batch_ragged")
     return T, dist, iters
 
 

@@ -278,6 +278,17 @@ int psd_icp_batch(const void *a, const void *b, int in_f64, int batch, int n, co
                   double tolerance, double *T_out, double *distances, int *iterations, void *stream);
 int psd_nn_f64(const void *src, const void *dst, int in_f64, int batch, int n_src, int n_dst, double *distances, int *indices,
                void *stream);
+/* The same for ragged batches: a [batch, n, 3] and b [batch, m, 3] are padded (fp32 or fp64 as in psd_icp_batch), and sample
+ * s aligns its first len_a[s] source points to its first len_b[s] destination points (device int [batch]; NULL = n / m),
+ * which need not be equal.  Points beyond the lengths are never read.  Outputs keep the padded shapes: distances
+ * [batch, n] is 0 beyond len_a[s].  A sample with a length outside [1, n] / [1, m] gets T all NaN, a NaN distance row and
+ * iterations -1, without affecting the others.  Each sample with len_a[s] == len_b[s] gives the bits of psd_icp_batch on
+ * its participating points alone.  The lengths are device data and are not read on the host (no synchronisation; capturable
+ * in a CUDA graph).  Returns -1 for batch < 0, n < 1, m < 1, n > 4096, n + m > 8192 or max_iterations < 1 (the
+ * max_iterations = 0 mode of psd_icp_batch needs equal sizes); otherwise as psd_icp_batch. */
+int psd_icp_batch_ragged(const void *a, const void *b, int in_f64, int batch, int n, int m, const int *len_a, const int *len_b,
+                         const double *init_pose, int max_iterations, double tolerance, double *T_out, double *distances,
+                         int *iterations, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * psd_farthest_point_sample  =  farthest_point_sample(xyz, npoint, RAN) of utils/utils.py:335-360 (called by the dataset
